@@ -19,9 +19,12 @@ for every problem, i.e. 4096 x 1000 inner Adam iterations per GPU per step.
              numpy restatement of it (oracle/linear_ref.py, bit-identical to it in the build
              container, kind "port" -- /root/reference does not exist on the GPU box); one
              single-threaded-BLAS process per host core, bounded sample.
-    parity_sample: 32 of the 4096 problems of the full default fit against the fits of the unmodified
-             reference recorded in tests/golden/fit_c4_sample32.npz (edge sets, |dW| next to the
+    parity_sample: 24 of the 4096 problems of the full default fit against the fits of the unmodified
+             reference recorded in tests/golden/fit_c4_sample24.npz (edge sets, |dW| next to the
              reference's own inv(M.T).T round-off envelope).
+    --dump-outputs DIR: what the last timed step returned, as DIR/<name>.npy (W of a fixed, seeded sample of
+             the problems, status and stage statistics of all of them), to compare two builds output for output;
+             the inputs depend only on the arguments.
     c5 / c2 / c3 / c1: the other configs of BASELINE.json (own roofline / e2e / CPU sample each);
     with --gpus N > 1 also the row-sharded C2 / C3 iterations and a strong-scaling C4 step.
 """
@@ -37,11 +40,15 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+# the bench leaves the tree as it found it (it may be read-only): no byte-code caches beside the sources, also in the
+# spawned CPU-baseline workers, which import this file first
+sys.dont_write_bytecode = True
 
 D, N_SAMPLES, K_EDGES = 64, 1000, 4
 LAMBDAS = (0.01, 0.02, 0.03, 0.05)
 ITERS_PER_STEP = 1000
 FLOP_PER_ITER = 4.0 * D ** 3
+DUMP_PROBLEMS = 512     # --dump-outputs: W of a fixed, seeded sample of the problems (512 x 64 x 64 float64 = 16.8 MB)
 
 
 # --------------------------------------------------------------------------- data
@@ -270,28 +277,28 @@ def traffic_from_profile(kernel: str):
 
 def parity_sample(W_raw, stage_iters):
     """The fitted W of the sampled problems of the 4096-batch against the full default fits of the UNMODIFIED
-    reference (tests/golden/fit_c4_sample32.npz, oracle/make_golden_scale.py c4): per-problem edge-set identity,
+    reference (tests/golden/fit_c4_sample24.npz, oracle/make_golden_scale.py c4): per-problem edge-set identity,
     |dW| next to the reference's own round-off envelope (the same fit with inv(M.T).T, SURVEY.md 7.4)."""
     import numpy as np
-    path = os.path.join(ROOT, "tests", "golden", "fit_c4_sample32.npz")
+    path = os.path.join(ROOT, "tests", "golden", "fit_c4_sample24.npz")
     if not os.path.exists(path):
         return None
     g = np.load(path)
     probs = [int(p) for p in g["problems"]]
     if max(probs) >= len(W_raw):
         return None
-    Wr, Wt = g["W_reference"], g["W_transposed"]
+    Wr = g["W_reference"]
     rows, n_same, n_env_same = [], 0, 0
     for k, p in enumerate(probs):
         W = W_raw[p]
-        e_gpu, e_ref, e_tr = np.abs(W) >= 0.3, np.abs(Wr[k]) >= 0.3, np.abs(Wt[k]) >= 0.3
+        e_gpu, e_ref = np.abs(W) >= 0.3, np.abs(Wr[k]) >= 0.3
         diff = int((e_gpu != e_ref).sum())
-        env_diff = int((e_tr != e_ref).sum())
+        env_diff = int(g["envelope_edge_diff"][k])
         n_same += diff == 0
         n_env_same += env_diff == 0
         ref_iters = [int(c[0]) for c in g["calls_reference"][k] if c[0] >= 0]
         row = {"problem": p, "edge_diff": diff, "max_abs_dW": float(np.abs(W - Wr[k]).max()),
-               "envelope_max_abs_dW": float(np.abs(Wt[k] - Wr[k]).max()), "envelope_edge_diff": env_diff,
+               "envelope_max_abs_dW": float(g["envelope_max_abs_dW"][k]), "envelope_edge_diff": env_diff,
                "stage_iters": [int(x) for x in stage_iters[p]], "reference_stage_iters": ref_iters}
         if diff:
             bad = np.argwhere(e_gpu != e_ref)
@@ -304,7 +311,7 @@ def parity_sample(W_raw, stage_iters):
             "max_abs_dW_median": float(np.median(dws)), "max_abs_dW_max": float(dws.max()),
             "envelope_median": float(np.median(envs)), "envelope_max": float(envs.max()),
             "same_stage_lengths": int(sum(r["stage_iters"] == r["reference_stage_iters"] for r in rows)),
-            "source": "tests/golden/fit_c4_sample32.npz (unmodified reference; envelope = the reference with inv(M.T).T)",
+            "source": "tests/golden/fit_c4_sample24.npz (unmodified reference; envelope = the reference with inv(M.T).T)",
             "per_problem": rows}
 
 
@@ -381,13 +388,14 @@ def bench_c5(torch, _lib, peak_tflops, with_cpu):
     gpath = os.path.join(ROOT, "tests", "golden", "fit_c5_reduced.npz")
     if os.path.exists(gpath):
         g = np.load(gpath)
-        W_ref = np.zeros(d * d)
-        W_ref[g["w_idx"]] = g["w_val"]
-        W_ref = W_ref.reshape(d, d)
-        big = np.abs(W_ref) >= 0.05
-        out["parity"] = {"edge_set_distance": int(((W_est != 0) != (np.abs(W_ref) >= 0.3)).sum()),
+        idx = np.cumsum(g["w_idx_delta"].astype(np.int64))         # flat indices of the entries |W_ref| >= 0.05
+        edges_ref = np.zeros(d * d, dtype=bool)
+        edges_ref[idx[g["w_edge"]]] = True
+        sample = idx[g["w_sample_pos"]]
+        out["parity"] = {"edge_set_distance": int(((W_est != 0).ravel() != edges_ref).sum()),
                          "edges": int((W_est != 0).sum()), "reference_edges": int(g["nnz_est"]),
-                         "max_abs_dW_on_ref_entries_ge_0.05": float(np.abs(model.W_raw - W_ref)[big].max()),
+                         "max_abs_dW_on_sampled_ref_entries_ge_0.05":
+                             float(np.abs(model.W_raw.ravel()[sample] - g["w_sample_val"]).max()),
                          "stage_iters": model.stage_iters, "reference_wall_s": float(g["wall_s"]),
                          "source": "tests/golden/fit_c5_reduced.npz (the same fit by the unmodified reference)"}
         out["e2e"]["speedup_vs_reference_fit_wall"] = float(g["wall_s"]) / wall
@@ -689,6 +697,18 @@ def bench_sharded(torch, dist, rank, world, dev):
     return out
 
 
+def dump_outputs(out_dir, res, W, rank, world):
+    """What the last timed step returned to its caller (W is updated in place), as float64 `out_dir/<name>.npy`:
+    W of a fixed, seeded sample of the problems, and status and stage statistics of every problem."""
+    import numpy as np
+    pick = np.sort(np.random.default_rng(0).choice(W.shape[0], min(DUMP_PROBLEMS, W.shape[0]), replace=False))
+    arrays = {"W_sample": W[pick.tolist()].cpu().numpy(), "W_sample_problems": pick.astype(np.float64),
+              "status": res.status.cpu().numpy().astype(np.float64), "stage_stats": res.stage_stats.cpu().numpy()}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + (f"_rank{rank}" if world > 1 else "") + ".npy"), a)
+
+
 def run_b200(args):
     import numpy as np
     import torch
@@ -747,6 +767,8 @@ def run_b200(args):
     kernel_ms = [ev[k].elapsed_time(ev[k + 1]) for k in range(args.steps)]
     done = sum(int(r.stage_stats[:, 0, 0].sum().item()) for r in results)
     assert done == nprob * ITERS_PER_STEP * args.steps, "a problem stopped early inside the timed region"
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, results[-1], W, rank, world)
 
     # ---- e2e: public host API, pinned host buffers, copies inside the timed region
     from midagma_b200 import minimize_batch
@@ -938,6 +960,8 @@ def main():
                     help="N > 1: skip the row-sharded C2 / C3 iterations")
     ap.add_argument("--extras-timeout", type=float, default=1500.0,
                     help="seconds after which the contract line is printed without the unfinished extra keys")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (float64, about 17 MB)")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)

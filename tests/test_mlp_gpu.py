@@ -4,6 +4,7 @@ import numpy as np
 import pytest
 import torch
 
+from oracle import simulate
 from oracle.nonlinear_ref import OracleMLP, OracleNonlinear
 
 pytestmark = pytest.mark.gpu
@@ -11,6 +12,11 @@ pytestmark = pytest.mark.gpu
 
 def _relmax(a, b):
     return np.abs(a - b).max() / max(np.abs(b).max(), 1e-300)
+
+
+def _checksum(a):
+    a = np.ascontiguousarray(a, dtype=np.float64)
+    return np.array([a.sum(), np.abs(a).sum(), (a * a).sum(), a.ravel()[:: max(a.size // 97, 1)].sum()])
 
 
 def _model_from(g, prefix="init."):
@@ -28,15 +34,25 @@ def test_mlp_value_grad_steps_vs_reference(golden, name):
     g = golden(name)
     lambda1, lambda2, mu, s, lr = (float(x) for x in g["hyper"])
     model = _model_from(g)
-    X = g["X"]
+    if "X" in g.files:
+        X, X_hat_ref = g["X"], g["X_hat"]
+    else:
+        # at n = 2000 the fixture keeps the seed of X (checksum of the arrays the reference was fed) and a fixed
+        # sample of the rows of X_hat
+        X, _ = simulate.config_c3(int(g["seed"]), n=int(g["n"]), d=int(g["dims"][0]))
+        assert np.allclose(_checksum(X), g["x_checksum"], rtol=1e-13, atol=0), "not the arrays the reference was fed"
+        X_hat_ref = None
+    rows = g["X_hat_rows"] if "X_hat_rows" in g.files else slice(None)
     # public surface: forward, h_func, l1, adjacency
-    assert _relmax(model.forward(torch.from_numpy(X)).numpy(), g["X_hat"]) <= 1e-12
+    X_hat = model.forward(torch.from_numpy(X))
+    assert _relmax(X_hat.numpy()[rows], g["X_hat"]) <= 1e-12
     assert abs(model.h_func(s).item() - float(g["h"])) <= 1e-9 * max(abs(float(g["h"])), 1e-3)
     assert _relmax(model.fc1_to_adj(), g["adj"]) <= 1e-13
     ref_l1 = np.abs(g["init.fc1.weight"]).sum()
     assert abs(model.fc1_l1_reg().item() - ref_l1) <= 1e-12 * ref_l1
     eq = DagmaNonlinear(model)
-    assert abs(eq.log_mse_loss(torch.from_numpy(g["X_hat"]), torch.from_numpy(X)).item() - float(g["score"])) \
+    X_hat = X_hat if X_hat_ref is None else torch.from_numpy(X_hat_ref)
+    assert abs(eq.log_mse_loss(X_hat, torch.from_numpy(X)).item() - float(g["score"])) \
         <= 1e-12 * abs(float(g["score"]))
     # one evaluation: objective pieces and every gradient within 1e-9 relative (north_star)
     eng = _MlpEngine(model, torch.from_numpy(X).cuda())
