@@ -102,6 +102,12 @@ typedef struct dagma_small_fit_args {
 } dagma_small_fit_args;
 
 int dagma_linear_fit_small_f64(dagma_stream_t stream, const dagma_small_fit_args* args);
+/* DagmaLinear('logistic').minimize / fit for a batch of problems; src/dagma/linear.py:90-92, 165-333, 441-457.
+ * args->cov_dev = X^T X / n of the UN-centred X; x_dev [batch][n][d] row-major; 1 <= d <= DAGMA_SMALL_MAX_D;
+ * args->ckpt_diag_dev must be NULL (no telemetry rows on this path).  One CTA per problem (two per SM), pulled
+ * from the work queue; X streams through shared memory every iteration.                                       */
+int dagma_linear_fit_small_logistic_f64(dagma_stream_t stream, const dagma_small_fit_args* args,
+                                        int n, const double* x_dev);
 /* launch geometry chosen for (d): CTAs, threads, dynamic shared memory bytes */
 int dagma_linear_fit_small_geometry(int d, int batch, int* ctas, int* threads, size_t* smem_bytes);
 

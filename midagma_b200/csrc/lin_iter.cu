@@ -36,6 +36,7 @@
 // stay on the launch sequence.
 #include "common.cuh"
 #include "small_dmma.cuh"
+#include "fit_step.cuh"
 #include "small_inv2.cuh"
 #include "gemm_f64.cuh"
 #include "lin_state.h"
@@ -353,9 +354,6 @@ __device__ __forceinline__ void li_stage_w(const LinIterArgs& P, const LiPlan& L
         }
     }
 }
-
-// 1 / (1 + exp(-z)) without the slow-path branches of the IEEE division (1 + e is in the normal range after the clamp)
-__device__ __forceinline__ double li_sigmoid(double z) { return fast_rcp(1.0 + exp(fmin(-z, 700.0))); }
 
 // ---------------------------------------------------------------- logistic worker: rows [c NR, (c + 1) NR) of X
 __device__ __forceinline__ void li_logistic_role(const LinIterArgs& P, const LiPlan& L, double* sm, int cta) {

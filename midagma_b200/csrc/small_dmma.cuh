@@ -398,13 +398,15 @@ struct ScoreFill {
 // ---------------------------------------------------------------- tensor memory (TMEM) scratch
 // Thread-private spill space: warp w owns TMEM lanes 32(w%4)..+31 (hardware rule for
 // tcgen05.ld/st), thread = lane; the two warps of a lane quarter use disjoint column ranges.
+template <int COLS = DM_TMEM_COLS>
 __device__ __forceinline__ void tmem_alloc(uint32_t smem_slot_addr) {   // one full warp
     asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_slot_addr),
-                 "n"(DM_TMEM_COLS) : "memory");
+                 "n"(COLS) : "memory");
     asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
 }
+template <int COLS = DM_TMEM_COLS>
 __device__ __forceinline__ void tmem_free(uint32_t taddr) {             // one full warp
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "n"(DM_TMEM_COLS) : "memory");
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "n"(COLS) : "memory");
 }
 __device__ __forceinline__ void tmem_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tmem_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }

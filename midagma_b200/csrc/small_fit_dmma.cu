@@ -19,9 +19,7 @@
 #endif
 #include "small_dmma.cuh"
 #include "small_fit_internal.h"
-#ifndef DAGMA_ADAM_GROUP
-#define DAGMA_ADAM_GROUP 4            // entries whose rsqrt / rcp Newton chains are interleaved in the element-wise pass
-#endif
+#include "fit_step.cuh"
 
 #ifndef DAGMA_FIT_GEMM_IN_SWEEP
 #define DAGMA_FIT_GEMM_IN_SWEEP 1     // 1: the score GEMM fills the waits of the sweep; 0: a separate phase after it
@@ -29,71 +27,6 @@
 #include "../../include/dagma_b200.h"
 
 namespace dagma {
-
-// c with the sign of w, 0 for w == +-0: c * sign(w) without touching the FP64 pipe
-__device__ __forceinline__ double signed_const(double w, double c) {
-    const int hi = __double2hiint(w), lo = __double2loint(w);
-    const bool zero = ((hi & 0x7fffffff) | lo) == 0;
-    const int chi = __double2hiint(c) ^ (hi & (int)0x80000000);
-    return zero ? 0.0 : __hiloint2double(chi, __double2loint(c));
-}
-
-// Scalar FP64 instructions are what the element-wise pass costs: with another CTA's DMMAs queued on the same FP64
-// pipe every one of them waits its turn (measured: 26 instructions per entry = 9.3 k clk per iteration with two CTAs
-// per SM, 3.5 k alone), so the pass is written for instruction count -- 20 per entry, none of them redundant:
-//   * moments are kept pre-divided by (1 - beta):  M = m / (1 - beta1), U = v / (1 - beta2), so that
-//       M <- beta1 M + g   (one fma),   U <- beta2 U + g^2   (one mul, one fma);
-//     mhat = M k1, vhat = U k2 with k1 = (1 - beta1) / (1 - beta1^it), k2 likewise            linear.py:158-161
-//   * sqrt(vhat): MUFU seed y ~ 1 / sqrt(x) (2^-22), s0 = x y, then two Heron steps s += (x - s^2) (y / 2) -- each two
-//     fmas, y / 2 by an exponent decrement: error 1.5 e^2 then 1.5 e^3, i.e. below one ulp
-//   * 1 / (s + 1e-8): MUFU seed + one Newton step, then the quotient is corrected by its own residual
-//   * 2 w by an exponent increment (w = +-0 stays), sign(w) constants by integer ops (signed_const)
-template <int N>
-__device__ __forceinline__ void adam_entries(double* __restrict__ w, const double* __restrict__ go, double* __restrict__ M,
-                                             double* __restrict__ U, double beta1, double beta2, double k1, double k2,
-                                             double lr) {
-    double x[N], y[N], hy[N], sq[N], dn[N], z[N];
-#pragma unroll
-    for (int q = 0; q < N; ++q) {
-        M[q] = fma(M[q], beta1, go[q]);
-        U[q] = fma(U[q], beta2, go[q] * go[q]);
-        x[q] = U[q] * k2;
-        asm("rsqrt.approx.ftz.f64 %0, %1;" : "=d"(y[q]) : "d"(x[q]));
-        const bool tiny = __double2hiint(x[q]) < 0x00200000;                 // vhat == 0 (or denormal): sqrt -> 0, not NaN
-        hy[q] = tiny ? 0.0 : __hiloint2double(__double2hiint(y[q]) - 0x00100000, __double2loint(y[q]));
-        if (tiny) y[q] = 0.0;
-        sq[q] = x[q] * y[q];
-    }
-#pragma unroll
-    for (int q = 0; q < N; ++q) sq[q] = fma(fma(-sq[q], sq[q], x[q]), hy[q], sq[q]);
-#pragma unroll
-    for (int q = 0; q < N; ++q) {
-        sq[q] = fma(fma(-sq[q], sq[q], x[q]), hy[q], sq[q]);
-        dn[q] = sq[q] + 1e-8;
-        asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(z[q]) : "d"(dn[q]));
-    }
-#pragma unroll
-    for (int q = 0; q < N; ++q) z[q] = fma(z[q], fma(-dn[q], z[q], 1.0), z[q]);
-#pragma unroll
-    for (int q = 0; q < N; ++q) {
-        const double mh = M[q] * k1;
-        const double qv = mh * z[q];
-        const double dir = fma(fma(-qv, dn[q], mh), z[q], qv);
-        w[q] = fma(-lr, dir, w[q]);
-    }
-}
-
-// 2 w without the FP64 pipe (w = +-0 and denormals are returned unchanged; |w| never gets near either overflow)
-__device__ __forceinline__ double twice(double w) {
-    const int hi = __double2hiint(w);
-    return __hiloint2double((hi & 0x7ff00000) ? hi + 0x00100000 : hi, __double2loint(w));
-}
-
-// a + 1e-16 < 0 for a finite a, as an integer comparison of the bit patterns (a < -1e-16 exactly: the sum is exact
-// near cancellation); keeps the sign test of linear.py:226-230 off the FP64 pipe
-__device__ __forceinline__ bool below_minus_1e16(double a) {
-    return (unsigned long long)__double_as_longlong(a) > 0xBC9CD2B297D889BCull;      // bits of -1e-16
-}
 
 #ifdef DAGMA_SWEEP_TRACE
 // debug build only: phase stamps of iteration 51 of CTA 0 -> rows 16.. of g_sweep_trace

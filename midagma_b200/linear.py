@@ -58,8 +58,9 @@ class SmallFitResult(typing.NamedTuple):
 
 def _run_small(cov: torch.Tensor, W: torch.Tensor, lambda1: torch.Tensor, mus, ss, iters, *, lr, tol,
                beta1, beta2, checkpoint, retry, mask_exc=None, mask_inc=None, ckpt_log_cap=0,
-               want_final=True, want_diag=False) -> SmallFitResult:
-    """Launch ``dagma_linear_fit_small_f64`` on device tensors (W is updated in place)."""
+               want_final=True, want_diag=False, X=None) -> SmallFitResult:
+    """Launch ``dagma_linear_fit_small_f64`` on device tensors (W is updated in place).  With ``X`` ([batch, n, d]
+    device tensor; ``cov`` = its un-centred X^T X / n) the logistic loss: ``dagma_linear_fit_small_logistic_f64``."""
     _lib.require_device()
     lib = _lib.load()
     batch, d, _ = cov.shape
@@ -67,7 +68,7 @@ def _run_small(cov: torch.Tensor, W: torch.Tensor, lambda1: torch.Tensor, mus, s
     if T > _lib.MAX_STAGES:
         return _run_small_chunked(cov, W, lambda1, mus, ss, iters, lr=lr, tol=tol, beta1=beta1, beta2=beta2,
                                   checkpoint=checkpoint, retry=retry, mask_exc=mask_exc, mask_inc=mask_inc,
-                                  ckpt_log_cap=ckpt_log_cap, want_final=want_final, want_diag=want_diag)
+                                  ckpt_log_cap=ckpt_log_cap, want_final=want_final, want_diag=want_diag, X=X)
     assert cov.is_cuda and W.is_cuda and cov.dtype == torch.float64 and W.dtype == torch.float64
     assert cov.is_contiguous() and W.is_contiguous() and lambda1.is_contiguous()
     dev = cov.device
@@ -96,7 +97,12 @@ def _run_small(cov: torch.Tensor, W: torch.Tensor, lambda1: torch.Tensor, mus, s
     a.ckpt_log = log.data_ptr() if log is not None else None
     a.ckpt_count = cnt.data_ptr() if cnt is not None else None
     a.work_counter = counter.data_ptr()
-    _lib.check(lib.dagma_linear_fit_small_f64(_lib.stream_ptr(), C.byref(a)), "dagma_linear_fit_small_f64")
+    if X is None:
+        _lib.check(lib.dagma_linear_fit_small_f64(_lib.stream_ptr(), C.byref(a)), "dagma_linear_fit_small_f64")
+    else:
+        assert X.is_cuda and X.dtype == torch.float64 and X.is_contiguous() and X.shape[0] == batch and X.shape[2] == d
+        _lib.check(lib.dagma_linear_fit_small_logistic_f64(_lib.stream_ptr(), C.byref(a), X.shape[1], X.data_ptr()),
+                   "dagma_linear_fit_small_logistic_f64")
     return SmallFitResult(W, status, stats, final, log, cnt, diag)
 
 
@@ -198,6 +204,23 @@ def _lam_dev(lambda1, batch: int, device) -> torch.Tensor:
     return _as_dev(np.broadcast_to(np.asarray(lambda1, dtype=np.float64), (batch,)), device)
 
 
+_LOSSES = ("l2", "logistic")
+
+
+def _logistic_inputs(loss_type, X, who: str) -> bool:
+    """Argument checks of the batched entry points that need no device; True for the logistic loss."""
+    if loss_type not in _LOSSES:
+        raise ValueError(f"{who}: loss_type should be one of {list(_LOSSES)}, got {loss_type!r}")
+    if loss_type == "l2":
+        return False
+    if X is None:
+        raise ValueError(f"{who}(loss_type='logistic') needs the data X [batch, n, d]: the logistic score is not a "
+                         "function of the covariance")
+    if np.ndim(X) != 3:
+        raise ValueError(f"{who}(loss_type='logistic'): X must be [batch, n, d], got shape {tuple(np.shape(X))}")
+    return True
+
+
 def _batch_masks(exclude_edges, include_edges, d, device):
     """Edge lists shared by the whole batch -> the [d, d] byte masks of the kernels.  Same acceptance rule as the
     reference (linear.py:416-426, Q5): anything but a tuple of 2-tuples is silently ignored."""
@@ -210,28 +233,35 @@ def _batch_masks(exclude_edges, include_edges, d, device):
 
 
 def minimize_batch(W, cov, lambda1, mu, max_iter, s, lr, *, tol=1e-6, beta_1=0.99, beta_2=0.999,
-                   checkpoint=1000, device=None, exclude_edges=None, include_edges=None):
-    """One ``DagmaLinear.minimize`` call (linear.py:165-333, l2 loss) for a batch of
+                   checkpoint=1000, device=None, exclude_edges=None, include_edges=None, loss_type="l2", X=None):
+    """One ``DagmaLinear(loss_type).minimize`` call (linear.py:165-333) for a batch of
     independent problems.  ``W``/``cov``: [batch, d, d] numpy arrays or torch tensors on
-    host (pinned or not) or device.  Like the reference, ``W`` is updated in place and
-    returned.  Returns ``(W, success[batch], stage_stats[batch, 1, 8])``."""
+    host (pinned or not) or device.  ``loss_type="logistic"`` needs the data ``X`` [batch, n, d]
+    (not centred, not modified); ``cov`` is then its X^T X / n and may be None (computed from X).
+    Like the reference, ``W`` is updated in place and returned.
+    Returns ``(W, success[batch], stage_stats[batch, 1, 8])``."""
+    logistic = _logistic_inputs(loss_type, X, "minimize_batch")
     _lib.require_device()
     device = torch.device(device or "cuda")
     on_device = isinstance(W, torch.Tensor) and W.is_cuda
-    if _host_pipeline_ok(W, cov):
+    if _host_pipeline_ok(W, cov, loss_type):
         return _minimize_batch_host_pipelined(W, cov, lambda1, mu, max_iter, s, lr, tol=tol, beta_1=beta_1, beta_2=beta_2,
                                               checkpoint=checkpoint, device=device, exclude_edges=exclude_edges,
                                               include_edges=include_edges)
     Wd = W if on_device and W.dtype == torch.float64 and W.is_contiguous() else _as_dev(W, device)
-    covd = _as_dev(cov, device)
+    Xd = _as_dev(X, device) if logistic else None
+    covd = center_cov(Xd, center=False) if logistic and cov is None else _as_dev(cov, device)
     batch, d, _ = covd.shape
+    if Xd is not None and (Xd.shape[0] != batch or Xd.shape[2] != d):
+        raise ValueError(f"minimize_batch: X {tuple(Xd.shape)} does not match W / cov [{batch}, {d}, {d}]")
     if d > _lib.SMALL_MAX_D:
         return _minimize_batch_large(W, covd, lambda1, mu, max_iter, s, lr, tol=tol, beta_1=beta_1, beta_2=beta_2,
-                                     checkpoint=checkpoint, exclude_edges=exclude_edges, include_edges=include_edges)
+                                     checkpoint=checkpoint, exclude_edges=exclude_edges, include_edges=include_edges,
+                                     Xd=Xd)
     lam = _lam_dev(lambda1, batch, device)
     mask_exc, mask_inc = _batch_masks(exclude_edges, include_edges, d, device)
     res = _run_small(covd, Wd, lam, [mu], [s], [int(max_iter)], lr=lr, tol=tol, beta1=beta_1, beta2=beta_2,
-                     checkpoint=checkpoint, retry=False, want_final=False, mask_exc=mask_exc, mask_inc=mask_inc)
+                     checkpoint=checkpoint, retry=False, want_final=False, mask_exc=mask_exc, mask_inc=mask_inc, X=Xd)
     ok = (res.status & _lib.ST_OUT_OF_DOMAIN) == 0
     if on_device:
         if Wd is not W:
@@ -247,10 +277,10 @@ def minimize_batch(W, cov, lambda1, mu, max_iter, s, lr, *, tol=1e-6, beta_1=0.9
 _COPY_STREAMS: dict = {}       # device index -> (H2D stream, D2H stream) of the pipelined host path
 
 
-def _host_pipeline_ok(W, cov) -> bool:
-    """Pinned host tensors of a batch that spans several waves of resident CTAs: worth overlapping the copies."""
+def _host_pipeline_ok(W, cov, loss_type="l2") -> bool:
+    """Pinned host tensors of an l2 batch that spans several waves of resident CTAs: worth overlapping the copies."""
     import os
-    if os.environ.get("DAGMA_HOST_PIPELINE", "1") == "0":
+    if loss_type != "l2" or os.environ.get("DAGMA_HOST_PIPELINE", "1") == "0":
         return False
     ok = all(isinstance(t, torch.Tensor) and not t.is_cuda and t.is_pinned() and t.dtype == torch.float64
              and t.is_contiguous() and t.dim() == 3 for t in (W, cov))
@@ -333,23 +363,31 @@ def _minimize_batch_host_pipelined(W, cov, lambda1, mu, max_iter, s, lr, *, tol,
 def fit_batch(X=None, lambda1=0.03, *, cov=None, w_threshold=0.3, T=5, mu_init=1.0, mu_factor=0.1,
               s=(1.0, .9, .8, .7, .6), warm_iter=3e4, max_iter=6e4, lr=0.0003, checkpoint=1000,
               beta_1=0.99, beta_2=0.999, tol=1e-6, device=None, return_info=False,
-              exclude_edges=None, include_edges=None):
-    """``DagmaLinear('l2').fit`` (linear.py:335-462) for a batch of independent problems.
+              exclude_edges=None, include_edges=None, loss_type="l2"):
+    """``DagmaLinear(loss_type).fit`` (linear.py:335-462) for a batch of independent problems.
 
-    ``X``: [batch, n, d] (centred on device, the caller's array is not modified) or
-    ``cov``: [batch, d, d].  ``lambda1``: scalar or [batch].  Each problem follows the
+    l2: ``X``: [batch, n, d] (centred on device, the caller's array is not modified) or
+    ``cov``: [batch, d, d].  logistic: ``X`` [batch, n, d] only (not centred, not modified; the
+    covariance is its X^T X / n).  ``lambda1``: scalar or [batch].  Each problem follows the
     reference schedule independently (own convergence checks, retries, back-tracking);
     problems are pulled from a device-side work queue by persistent CTAs.
     ``exclude_edges`` / ``include_edges``: tuples of 2-tuples shared by the batch (linear.py:416-426).
     Returns thresholded ``W_est`` [batch, d, d] as numpy (+ info dict)."""
+    logistic = _logistic_inputs(loss_type, X, "fit_batch")
+    if logistic and cov is not None:
+        raise ValueError("fit_batch(loss_type='logistic') takes X only: the covariance is computed from it")
     _lib.require_device()
     device = torch.device(device or "cuda")
-    if cov is None:
+    Xd = None
+    if logistic:
         Xd = _as_dev(X, device)
-        if Xd.data_ptr() == (X.data_ptr() if isinstance(X, torch.Tensor) else 0):
-            Xd = Xd.clone()
-        covd = center_cov(Xd, center=True)
-        del Xd
+        covd = center_cov(Xd, center=False)
+    elif cov is None:
+        Xc = _as_dev(X, device)
+        if Xc.data_ptr() == (X.data_ptr() if isinstance(X, torch.Tensor) else 0):
+            Xc = Xc.clone()
+        covd = center_cov(Xc, center=True)
+        del Xc
     else:
         covd = _as_dev(cov, device)
     batch, d, _ = covd.shape
@@ -357,7 +395,7 @@ def fit_batch(X=None, lambda1=0.03, *, cov=None, w_threshold=0.3, T=5, mu_init=1
         return _fit_batch_large(covd, lambda1, w_threshold=w_threshold, T=T, mu_init=mu_init, mu_factor=mu_factor, s=s,
                                 warm_iter=warm_iter, max_iter=max_iter, lr=lr, checkpoint=checkpoint, beta_1=beta_1,
                                 beta_2=beta_2, return_info=return_info, exclude_edges=exclude_edges,
-                                include_edges=include_edges)
+                                include_edges=include_edges, Xd=Xd)
     lam = _lam_dev(lambda1, batch, device)
     T = int(T)
     ss = list(s) if isinstance(s, (list, tuple)) else T * [s]
@@ -368,7 +406,7 @@ def fit_batch(X=None, lambda1=0.03, *, cov=None, w_threshold=0.3, T=5, mu_init=1
     Wd = torch.zeros(batch, d, d, dtype=torch.float64, device=device)
     mask_exc, mask_inc = _batch_masks(exclude_edges, include_edges, d, device)
     res = _run_small(covd, Wd, lam, mus, ss[:T], iters, lr=lr, tol=tol, beta1=beta_1, beta2=beta_2,
-                     checkpoint=checkpoint, retry=True, mask_exc=mask_exc, mask_inc=mask_inc)
+                     checkpoint=checkpoint, retry=True, mask_exc=mask_exc, mask_inc=mask_inc, X=Xd)
     _warn_retry_limit(res.status)
     W_raw = res.W.cpu().numpy()
     W_est = W_raw.copy()
@@ -383,9 +421,10 @@ def fit_batch(X=None, lambda1=0.03, *, cov=None, w_threshold=0.3, T=5, mu_init=1
     return W_est, info
 
 
-def _batch_lanes(d: int, batch: int) -> int:
+def _batch_lanes(d: int, batch: int, n: typing.Optional[int] = None) -> int:
     """How many problems of a d > 64 batch run side by side.  For d <= 128 a problem's inner iterations are one
-    persistent kernel of ceil(d / 8) + 1 CTAs (csrc/lin_iter.cu), each alone on its SM, so several problems fit on the
+    persistent kernel (csrc/lin_iter.cu) of ceil(d / 8) + 1 CTAs for l2, and for the logistic loss (``n`` rows of X)
+    of one CTA per block of rows plus the inverse CTA, each alone on its SM, so several problems fit on the
     device at once -- one host thread and one CUDA stream per lane (DAGMA_BATCH_LANES overrides; 1 = one after the
     other).  Beyond d = 128 the blocked inverse fills the device by itself."""
     import os
@@ -393,20 +432,28 @@ def _batch_lanes(d: int, batch: int) -> int:
     if env:
         return max(1, min(int(env), batch))
     lib = _lib.load()
-    if d > 128 or not lib.dagma_linear_iter_supported(0, 0, d) or os.environ.get("DAGMA_LIN_FUSED", "1") == "0":
+    logistic = n is not None
+    if (d > 128 or not lib.dagma_linear_iter_supported(int(logistic), n or 0, d)
+            or os.environ.get("DAGMA_LIN_FUSED", "1") == "0"):
         return 1
     sms = torch.cuda.get_device_properties(torch.cuda.current_device()).multi_processor_count
-    ctas = (d + 7) // 8 + 1
+    if logistic:
+        # li_plan: the rows are spread over the SMs but one, in blocks of a multiple of 8 rows per worker CTA
+        per = -(-n // (sms - 1))
+        rows = 8 * -(-per // 8)
+        ctas = -(-n // rows) + 1
+    else:
+        ctas = (d + 7) // 8 + 1
     return max(1, min((sms - 12) // ctas, 8, batch))       # a dozen SMs stay free for the checkpoint kernels of all lanes
 
 
 _LANE_STREAMS: dict = {}       # device index -> raw streams of the batch lanes (created once, reused)
 
 
-def _run_lanes(batch: int, d: int, solve, device) -> None:
+def _run_lanes(batch: int, d: int, solve, device, n: typing.Optional[int] = None) -> None:
     """``solve(b)`` for every problem of a d > 64 batch, ``_batch_lanes`` of them at a time: one host thread and one
     CUDA stream per lane (the caller's stream is waited for first; every lane is synchronised before returning)."""
-    lanes = _batch_lanes(d, batch)
+    lanes = _batch_lanes(d, batch, n)
     if lanes <= 1:
         for b in range(batch):
             solve(b)
@@ -454,7 +501,7 @@ def _run_lanes(batch: int, d: int, solve, device) -> None:
 
 
 def _minimize_batch_large(W, covd, lambda1, mu, max_iter, s, lr, *, tol, beta_1, beta_2, checkpoint, exclude_edges,
-                          include_edges):
+                          include_edges, Xd=None):
     """``minimize_batch`` beyond the on-chip size: one ``DagmaLinear.minimize`` per problem on the multi-CTA engine, for
     d <= 128 several problems side by side (one persistent kernel each, csrc/lin_iter.cu)."""
     batch, d, _ = covd.shape
@@ -466,16 +513,17 @@ def _minimize_batch_large(W, covd, lambda1, mu, max_iter, s, lr, *, tol, beta_1,
     stats = np.zeros((batch, 1, 8))
 
     def solve(b):
-        m = DagmaLinear("l2")
+        m = DagmaLinear("l2" if Xd is None else "logistic")
         m._fit_from_cov(covd[b], float(lam[b]), T=1, warm_iter=0, max_iter=0, checkpoint=checkpoint,
-                        exclude_edges=exclude_edges, include_edges=include_edges)
+                        exclude_edges=exclude_edges, include_edges=include_edges,
+                        X_dev=Xd[b] if Xd is not None else None)
         _, ok[b] = m.minimize(W_out[b], mu, int(max_iter), s, lr=lr, tol=tol, beta_1=beta_1, beta_2=beta_2)
         stats[b, 0, 0] = m.last_iters
         stats[b, 0, 1], stats[b, 0, 2] = m._large.last_lr, s
         if m.checkpoint_log:
             stats[b, 0, 3:6] = m.checkpoint_log[-1][2:5]
 
-    _run_lanes(batch, d, solve, covd.device)
+    _run_lanes(batch, d, solve, covd.device, Xd.shape[1] if Xd is not None else None)
     if isinstance(W, torch.Tensor):
         W.copy_(torch.from_numpy(W_out))
         return W, (torch.from_numpy(ok).to(W.device) if W.is_cuda else ok), (torch.from_numpy(stats).to(W.device) if W.is_cuda else stats)
@@ -483,7 +531,7 @@ def _minimize_batch_large(W, covd, lambda1, mu, max_iter, s, lr, *, tol, beta_1,
     return W, ok, stats
 
 
-def _fit_batch_large(covd, lambda1, *, w_threshold, return_info, **fit_kw):
+def _fit_batch_large(covd, lambda1, *, w_threshold, return_info, Xd=None, **fit_kw):
     """``fit_batch`` beyond the on-chip size (d > 64): every problem runs on the multi-CTA engine -- the same code path
     as ``DagmaLinear.fit`` at that size, fed with the covariance instead of the data -- and ``_batch_lanes`` problems
     run concurrently, each on its own stream (for d <= 128 the inner iterations of a problem are one persistent kernel
@@ -495,14 +543,14 @@ def _fit_batch_large(covd, lambda1, *, w_threshold, return_info, **fit_kw):
     stage_iters, h_fin, sc_fin = [None] * batch, [None] * batch, [None] * batch
 
     def solve(b):
-        m = DagmaLinear("l2")
+        m = DagmaLinear("l2" if Xd is None else "logistic")
         kw = dict(fit_kw)
         kw["s"] = list(kw["s"]) if isinstance(kw["s"], (list, tuple)) else kw["s"]
-        m._fit_from_cov(covd[b], float(lam[b]), **kw)
+        m._fit_from_cov(covd[b], float(lam[b]), X_dev=Xd[b] if Xd is not None else None, **kw)
         W_raw[b] = m.W_raw
         stage_iters[b], h_fin[b], sc_fin[b] = m.stage_iters, m.h_final, m.score_final
 
-    _run_lanes(batch, d, solve, covd.device)
+    _run_lanes(batch, d, solve, covd.device, Xd.shape[1] if Xd is not None else None)
     W_est = W_raw.copy()
     W_est[np.abs(W_est) < w_threshold] = 0
     if not return_info:
@@ -739,15 +787,16 @@ class DagmaLinear:
 
     def _fit_from_cov(self, cov_dev: torch.Tensor, lambda1: float, *, T=5, mu_init=1.0, mu_factor=0.1,
                       s=(1.0, .9, .8, .7, .6), warm_iter=3e4, max_iter=6e4, lr=0.0003, checkpoint=1000, beta_1=0.99,
-                      beta_2=0.999, exclude_edges=None, include_edges=None) -> np.ndarray:
-        """The path-following loop of ``fit`` (l2) from a device covariance instead of the data (batched entry point)."""
-        assert self.loss_type == 'l2'
+                      beta_2=0.999, exclude_edges=None, include_edges=None, X_dev=None) -> np.ndarray:
+        """The path-following loop of ``fit`` from a device covariance instead of the data (batched entry points);
+        the logistic loss also needs the data itself, ``X_dev`` [n, d] on the device (cov = X^T X / n, un-centred)."""
+        assert self.loss_type == 'l2' or X_dev is not None
         self.X, self.lambda1, self.checkpoint = None, lambda1, checkpoint
         self.d = int(cov_dev.shape[0])
-        self.n = self._n_total = 0
+        self.n = self._n_total = int(X_dev.shape[0]) if X_dev is not None else 0
         self.Id = np.eye(self.d).astype(self.dtype)
         self.checkpoint_log = []
-        self._X_dev = None
+        self._X_dev = X_dev.contiguous() if X_dev is not None else None
         self._cov_dev = cov_dev.contiguous()
         self.cov = self._cov_dev.cpu().numpy()
         self._run_path(lambda1, T, mu_init, mu_factor, s, warm_iter, max_iter, lr, checkpoint, beta_1, beta_2,
