@@ -74,11 +74,17 @@ extern "C" int dagma_center_cov_f64(dagma_stream_t stream_, int batch, int n, in
     DAGMA_REQUIRE(x_dev && cov_dev, "null pointer");
     cudaStream_t stream = (cudaStream_t)stream_;
     const int tiles = (d + 31) / 32;
-    if (center) {
-        center_columns_kernel<<<dim3(tiles, batch), dim3(32, 8), 0, stream>>>(x_dev, n, d);
+    // the problems sit on gridDim.y / gridDim.z, which CUDA caps at 65 535: larger batches go in slices
+    constexpr int kMaxGridYZ = 65535;
+    for (int b0 = 0; b0 < batch; b0 += kMaxGridYZ) {
+        const int nb = batch - b0 < kMaxGridYZ ? batch - b0 : kMaxGridYZ;
+        double* x = x_dev + (size_t)b0 * n * d;
+        if (center) {
+            center_columns_kernel<<<dim3(tiles, nb), dim3(32, 8), 0, stream>>>(x, n, d);
+            DAGMA_CUDA_OK(cudaGetLastError());
+        }
+        cov_kernel<<<dim3(tiles, tiles, nb), dim3(16, 16), 0, stream>>>(x, cov_dev + (size_t)b0 * d * d, n, d, 0, n);
         DAGMA_CUDA_OK(cudaGetLastError());
     }
-    cov_kernel<<<dim3(tiles, tiles, batch), dim3(16, 16), 0, stream>>>(x_dev, cov_dev, n, d, 0, n);
-    DAGMA_CUDA_OK(cudaGetLastError());
     return 0;
 }
