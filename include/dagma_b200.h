@@ -292,6 +292,21 @@ int dagma_mlp_iter_sharded_f64(dagma_stream_t stream, int n_local, int n_total, 
                                void* state_dev, double* theta_dev, double* m_dev, double* v_dev, const double* x_dev,
                                double* part_dev, double* minv_dev, unsigned* sync_dev, int rank, int nranks,
                                void* const* exchange_ptrs);
+/* Batched DagmaNonlinear.minimize (nonlinear.py:161-236, one call per problem) for many independent dims = [d, m1, 1]
+ * problems of the same shape, ONE CTA per problem from a work queue (csrc/mlp_batch.cu).  Problem b runs up to
+ * max_iter iterations from states_dev[b] (MlpState: mu, s, lr, lambda1, lambda2, beta1, beta2, lr_gamma, step and
+ * halted are read; lr, logabsdet, h, S, l1, obj, score, step and halted are written), theta/m/v [batch][W] with
+ * W = d*m1*d + 2*d*m1 + d (the layout above) and x_dev [batch][n][d]; it stops at h < 0 (halted = 1: the reference
+ * returns False, nonlinear.py:215-217) or when the objective meets tol at a checkpoint iteration
+ * (i % checkpoint == 0 or i == max_iter - 1, nonlinear.py:226-231).  idx_dev (optional): the n_idx problems to
+ * run; NULL runs all of them.  grad_dev [batch][W]: scratch; iters_dev[b]: the iterations run;
+ * work_counter_dev: one uint32.
+ *   supported : 1 when 1 <= d <= 64, 1 <= m1 <= 40 and n >= 1                                               */
+int dagma_mlp_batch_supported(int n, int d, int m1);
+int dagma_mlp_minimize_batch_f64(dagma_stream_t stream, int batch, int n, int d, int m1, int max_iter, int checkpoint,
+                                 double tol, const int* idx_dev, int n_idx, void* states_dev, double* theta_dev,
+                                 double* m_dev, double* v_dev, const double* x_dev, double* grad_dev, int* iters_dev,
+                                 unsigned* work_counter_dev);
 /* General LocallyConnected stacks dims = [d, m_1, ..., 1] (nonlinear.py:39-43, 60-65), transposed activations
  * [d * width][n], one call per layer.
  *   lc_forward : in ([d*mi][n]; + bias_in for the first layer) is replaced by H = sigmoid(in);

@@ -110,7 +110,11 @@ EXPORTS = {
     "dagma_mlp_iter_sharded_f64": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
                                              C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                              C.c_int, C.c_int, C.c_void_p]),
-    "dagma_lc_forward_f64": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+    "dagma_mlp_batch_supported": (C.c_int, [C.c_int, C.c_int, C.c_int]),
+    "dagma_mlp_minimize_batch_f64": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
+                                               C.c_double, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+                                               C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "dagma_lc_forward_f64":(C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
                                        C.c_void_p, C.c_void_p]),
     "dagma_mlp_residual_f64": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                          C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),

@@ -12,6 +12,9 @@ synchronises at the convergence checkpoints.  ``dims = [d, m1, 1]`` (the referen
 BASELINE.json's configuration) runs on fused forward / backward kernels; any other stack
 ``[d, m1, ..., 1]`` (and the degenerate ``[d, 1]``) runs layer by layer on the generic
 LocallyConnected kernels.
+
+``fit_batch`` / ``minimize_batch`` run many independent ``[d, m1, 1]`` problems of one shape (d <= 64, m1 <= 40) in
+one launch, one CTA per problem (csrc/mlp_batch.cu); other shapes run one ``DagmaNonlinear`` after the other.
 """
 from __future__ import annotations
 
@@ -25,7 +28,7 @@ import torch.nn as nn
 from . import _lib
 from ._large import gemm
 
-__all__ = ["DagmaMLP", "DagmaNonlinear", "LocallyConnected"]
+__all__ = ["DagmaMLP", "DagmaNonlinear", "LocallyConnected", "fit_batch", "minimize_batch"]
 
 ST_DOUBLES = 17
 (F_MU, F_S, F_LR, F_LAM1, F_LAM2, F_B1, F_B2, F_LAD, F_H, F_MIN, F_SS, F_L1, F_OBJ, F_SCORE, F_GAMMA) = range(15)
@@ -528,3 +531,184 @@ class DagmaNonlinear:
         W_est = self.model.fc1_to_adj()
         W_est[np.abs(W_est) < w_threshold] = 0
         return W_est
+
+
+# ------------------------------------------------------------------------------------------------ batched problems
+def _batch_inputs(models, X, fname):
+    if not isinstance(models, (list, tuple)) or len(models) == 0:
+        raise ValueError(f"{fname}: models must be a non-empty list of DagmaMLP")
+    dims = list(models[0].dims)
+    if any(list(m.dims) != dims for m in models):
+        raise ValueError(f"{fname}: every model must have the same dims (got {dims} and others)")
+    if isinstance(X, np.ndarray):
+        X = torch.from_numpy(X)
+    if not isinstance(X, torch.Tensor) or X.dim() != 3 or X.shape[0] != len(models) or X.shape[2] != dims[0]:
+        raise ValueError(f"{fname}: X must be [batch, n, d] = [{len(models)}, n, {dims[0]}], "
+                         f"got {tuple(X.shape) if hasattr(X, 'shape') else type(X)}")
+    if X.shape[1] < 1:
+        raise ValueError(f"{fname}: X has no rows")
+    return dims, X
+
+
+def _per_problem(x, batch, name):
+    a = np.asarray(x, dtype=np.float64)
+    if a.ndim == 0:
+        return np.full(batch, float(a))
+    if a.shape != (batch,):
+        raise ValueError(f"{name} must be a scalar or [{batch}], got shape {a.shape}")
+    return a.copy()
+
+
+class _MlpBatch:
+    """Device buffers of a batch of [d, m1, 1] problems on the one-CTA-per-problem kernel (csrc/mlp_batch.cu)."""
+
+    def __init__(self, models, X: torch.Tensor):
+        self.lib = _lib.load()
+        self.models = models
+        self.B, self.n, self.d = X.shape
+        self.m1 = int(models[0].dims[1])
+        self.X = _cuda64(X)
+        self.theta = torch.stack([m.pack() for m in models])
+        self.W = self.theta.shape[1]
+        self.m = torch.zeros_like(self.theta)
+        self.v = torch.zeros_like(self.theta)
+        self.grad = torch.empty_like(self.theta)
+        self.state = torch.zeros(self.B, ST_DOUBLES, dtype=torch.float64, device="cuda")
+        self.iters = torch.zeros(self.B, dtype=torch.int32, device="cuda")
+        self.counter = torch.zeros(1, dtype=torch.int32, device="cuda")
+
+    def run(self, idx, max_iter, lr, lambda1, lambda2, mu, s, lr_decay, tol, checkpoint):
+        """One minimize call (fresh Adam state) for the problems `idx`; per-problem arrays are indexed by problem.
+        Returns (success, iterations) of those problems."""
+        idx = np.asarray(idx, dtype=np.int64)
+        if idx.size == 0:
+            return np.zeros(0, dtype=bool), np.zeros(0, dtype=np.int64)
+        sh = np.zeros((idx.size, ST_DOUBLES))
+        for f, val in ((F_MU, mu), (F_S, s), (F_LR, lr), (F_LAM1, lambda1), (F_LAM2, lambda2)):
+            sh[:, f] = np.asarray(val, dtype=np.float64)[idx]
+        sh[:, F_B1], sh[:, F_B2] = 0.99, 0.999
+        sh[:, F_GAMMA] = np.where(np.asarray(lr_decay)[idx], 0.8, 1.0)
+        rows = torch.from_numpy(idx).cuda()
+        self.state[rows] = torch.from_numpy(sh).cuda()          # step = halted = 0
+        self.m[rows] = 0.0                                     # optimizer re-created per call (Q13)
+        self.v[rows] = 0.0
+        full = idx.size == self.B and np.array_equal(idx, np.arange(self.B))
+        idx_dev = None if full else rows.to(torch.int32)
+        _lib.check(self.lib.dagma_mlp_minimize_batch_f64(
+            _lib.stream_ptr(), self.B, self.n, self.d, self.m1, int(max_iter), int(checkpoint), float(tol),
+            idx_dev.data_ptr() if idx_dev is not None else None, int(idx.size), self.state.data_ptr(),
+            self.theta.data_ptr(), self.m.data_ptr(), self.v.data_ptr(), self.X.data_ptr(), self.grad.data_ptr(),
+            self.iters.data_ptr(), self.counter.data_ptr()), "dagma_mlp_minimize_batch_f64")
+        halted = self.state[:, 15:].contiguous().view(torch.int32)[:, I_HALTED]
+        ok = (halted[rows] == 0).cpu().numpy()
+        return ok, self.iters[rows].cpu().numpy().astype(np.int64)
+
+    def write_back(self):
+        for b, model in enumerate(self.models):
+            model.unpack(self.theta[b])
+
+
+def _supported(dims, n) -> bool:
+    return len(dims) == 3 and bool(_lib.load().dagma_mlp_batch_supported(int(n), int(dims[0]), int(dims[1])))
+
+
+@torch.no_grad()
+def minimize_batch(models, X, max_iter, lr, lambda1, lambda2, mu, s, lr_decay=False, tol=1e-6,
+                   checkpoint=1000) -> np.ndarray:
+    """``DagmaNonlinear(model).minimize(...)`` for every model, with ``X[b]`` as that model's data
+    (nonlinear.py:161-236).  ``models``: DagmaMLP objects of identical ``dims``, updated in place; ``X``: [batch, n, d]
+    (host or device, not modified); ``lambda1`` / ``lambda2``: scalar or [batch].  Returns ``success`` [batch].
+    ``[d, m1, 1]`` with d <= 64, m1 <= 40 runs in one launch (csrc/mlp_batch.cu); other shapes one model at a time."""
+    dims, X = _batch_inputs(models, X, "minimize_batch")
+    B, n = X.shape[0], X.shape[1]
+    lam1, lam2 = _per_problem(lambda1, B, "lambda1"), _per_problem(lambda2, B, "lambda2")
+    _lib.require_device()
+    if not _supported(dims, n):
+        out = np.zeros(B, dtype=bool)
+        for b, model in enumerate(models):
+            eq = DagmaNonlinear(model)
+            eq.X, eq.checkpoint = _cuda64(X[b]), checkpoint
+            out[b] = eq.minimize(max_iter, lr, float(lam1[b]), float(lam2[b]), mu, s, lr_decay, tol)
+        return out
+    bt = _MlpBatch(models, X)
+    full = lambda x: np.full(B, x)                              # noqa: E731
+    ok, _ = bt.run(np.arange(B), int(max_iter), full(float(lr)), lam1, lam2, full(float(mu)), full(float(s)),
+                   full(lr_decay is True), tol, checkpoint)
+    bt.write_back()
+    return ok
+
+
+@torch.no_grad()
+def fit_batch(models, X, lambda1=.02, lambda2=.005, T=4, mu_init=.1, mu_factor=.1, s=1.0, warm_iter=5e4, max_iter=8e4,
+              lr=2e-4, w_threshold=.3, checkpoint=1000, return_info=False, device=None):
+    """``DagmaNonlinear(model).fit(X[b], ...)`` for every model (nonlinear.py:486-530): the same stage loop per
+    problem -- a failed minimize restores the stage-start parameters, halves that problem's lr (for the rest of its
+    fit), turns on ExponentialLR and retries with s = 1 -- with every minimize call of a stage run for all problems in
+    one launch and the retries relaunched for the failed problems only.  ``models`` are updated in place; returns
+    W_est [batch, d, d] and, with ``return_info``, a dict of ``W_raw``, ``stage_iters`` (the iterations of each stage's
+    last minimize call), ``n_iters`` (of every call) and ``minimize_calls`` (per problem, (lr, s, success, lr_decay)
+    of every call), as DagmaNonlinear keeps them.  ``device``: the CUDA device to run on (default: the current one)."""
+    if device is not None:
+        with torch.cuda.device(torch.device(device)):
+            return fit_batch(models, X, lambda1, lambda2, T, mu_init, mu_factor, s, warm_iter, max_iter, lr,
+                             w_threshold, checkpoint, return_info)
+    dims, X = _batch_inputs(models, X, "fit_batch")
+    B, n = X.shape[0], X.shape[1]
+    lam1, lam2 = _per_problem(lambda1, B, "lambda1"), _per_problem(lambda2, B, "lambda2")
+    T = int(T)
+    if isinstance(s, list):
+        s = s + (T - len(s)) * [s[-1]] if len(s) < T else s
+    elif isinstance(s, (int, float)):
+        s = T * [s]
+    else:
+        raise ValueError("s should be a list, int, or float.")
+    _lib.require_device()
+    if not _supported(dims, n):
+        eqs = []
+        for b, model in enumerate(models):
+            eq = DagmaNonlinear(model)
+            eq.fit(X[b], lambda1=float(lam1[b]), lambda2=float(lam2[b]), T=T, mu_init=mu_init, mu_factor=mu_factor,
+                   s=list(s), warm_iter=warm_iter, max_iter=max_iter, lr=lr, w_threshold=w_threshold,
+                   checkpoint=checkpoint)
+            eqs.append(eq)
+        stage_iters = [list(eq.stage_iters) for eq in eqs]
+        calls = [list(eq.minimize_calls) for eq in eqs]
+        n_iters = np.array([eq.n_iters for eq in eqs], dtype=np.int64)
+    else:
+        bt = _MlpBatch(models, X)
+        lr_b = np.full(B, float(lr))
+        n_iters = np.zeros(B, dtype=np.int64)
+        stage_iters = [[] for _ in range(B)]
+        calls = [[] for _ in range(B)]
+        mu = mu_init
+        for i in range(T):
+            inner = int(max_iter) if i == T - 1 else int(warm_iter)
+            snap = bt.theta.clone()
+            s_cur = np.full(B, float(s[i]))
+            decay = np.zeros(B, dtype=bool)
+            last = np.zeros(B, dtype=np.int64)
+            todo = np.arange(B)
+            while todo.size:
+                ok, its = bt.run(todo, inner, lr_b, lam1, lam2, np.full(B, float(mu)), s_cur, decay, 1e-6, checkpoint)
+                n_iters[todo] += its
+                last[todo] = its
+                for b, good in zip(todo, ok):
+                    calls[b].append((float(lr_b[b]), float(s_cur[b]), int(good), int(decay[b])))
+                failed = todo[~ok]
+                if failed.size:
+                    rows = torch.from_numpy(failed).cuda()
+                    bt.theta[rows] = snap[rows]
+                    lr_b[failed] *= 0.5
+                    decay[failed] = True
+                    s_cur[failed] = 1.0
+                todo = failed[lr_b[failed] >= 1e-10]
+            for b in range(B):                     # the stage's last minimize call, as DagmaNonlinear.fit counts it
+                stage_iters[b].append(int(last[b]))
+            mu *= mu_factor
+        bt.write_back()
+    W_raw = np.stack([model.fc1_to_adj() for model in models])
+    W_est = W_raw.copy()
+    W_est[np.abs(W_est) < w_threshold] = 0
+    if not return_info:
+        return W_est
+    return W_est, {"W_raw": W_raw, "stage_iters": stage_iters, "n_iters": n_iters, "minimize_calls": calls}
