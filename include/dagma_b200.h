@@ -125,7 +125,9 @@ int dagma_linear_fit_small_host_f64(dagma_stream_t stream, const dagma_small_fit
  * sigmoid epilogue (epilogue = 1).  Replaces the BLAS calls of the score:
  *   cov @ (I - W)                       src/dagma/linear.py:86, 244
  *   X @ W, (X^T / n) @ sigmoid(X @ W)   src/dagma/linear.py:90-92, 246
- * ws_dev: optional split-K workspace (deterministic two-pass reduction).              */
+ * ws_dev: optional split-K workspace (deterministic two-pass reduction).
+ * lda >= K (trans_a: lda >= M), ldb >= N, ldc >= N; K = 0 gives C = beta * C (then the
+ * epilogue), as BLAS does.                                                            */
 int dagma_gemm_f64(dagma_stream_t stream, int trans_a, int M, int N, int K, double alpha,
                    const double* a_dev, int lda, const double* b_dev, int ldb, double beta,
                    double* c_dev, int ldc, int epilogue, double* ws_dev, size_t ws_bytes);

@@ -54,8 +54,9 @@ static int gemm_launch_tile(cudaStream_t stream, int transA, int M, int N, int K
         while (splits > 1 && (size_t)splits * M * N * sizeof(double) > ws_bytes) --splits;
         if (splits < 1) splits = 1;
     }
-    int kchunk_tiles = (ktiles + splits - 1) / splits;
-    splits = (ktiles + kchunk_tiles - 1) / kchunk_tiles;
+    // K = 0: one pass with an empty k range, so the kernel's epilogue leaves beta * C (and the sigmoid), as BLAS does
+    const int kchunk_tiles = ktiles > 0 ? (ktiles + splits - 1) / splits : 1;
+    splits = ktiles > 0 ? (ktiles + kchunk_tiles - 1) / kchunk_tiles : 1;
     GemmArgs P{M, N, K, A, lda, B, ldb, C, ldc, alpha, beta, kchunk_tiles * GBK, splits > 1 ? ws : nullptr};
     dim3 grid(tn, tm, splits);
     const size_t sm = T::SMEM_BYTES;
@@ -2465,9 +2466,10 @@ extern "C" int dagma_gemm_f64(dagma_stream_t stream, int trans_a, int M, int N, 
                               const double* a_dev, int lda, const double* b_dev, int ldb, double beta,
                               double* c_dev, int ldc, int epilogue, double* ws_dev, size_t ws_bytes) {
     DAGMA_REQUIRE(a_dev && b_dev && c_dev, "null pointer");
-    DAGMA_REQUIRE(K >= 0 && lda >= 1 && ldb >= N && ldc >= N, "bad leading dimension");
-    return gemm_launch((cudaStream_t)stream, trans_a, M, N, K, alpha, a_dev, lda, b_dev, ldb, beta, c_dev, ldc,
-                       epilogue, ws_dev, ws_bytes);
+    DAGMA_REQUIRE(K >= 0 && lda >= 1 && lda >= (trans_a ? M : K) && ldb >= N && ldc >= N, "bad leading dimension");
+    // K = 0: C = beta C (then the epilogue) whatever alpha is -- alpha times the empty sum would be NaN for alpha = inf
+    return gemm_launch((cudaStream_t)stream, trans_a, M, N, K, K > 0 ? alpha : 0.0, a_dev, lda, b_dev, ldb, beta, c_dev,
+                       ldc, epilogue, ws_dev, ws_bytes);
 }
 
 extern "C" int dagma_logdet_inv_ws_f64(dagma_stream_t stream, int d, double s, const double* a_dev, int lda,
