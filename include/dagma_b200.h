@@ -108,6 +108,21 @@ int dagma_linear_fit_small_f64(dagma_stream_t stream, const dagma_small_fit_args
  * from the work queue; X streams through shared memory every iteration.                                       */
 int dagma_linear_fit_small_logistic_f64(dagma_stream_t stream, const dagma_small_fit_args* args,
                                         int n, const double* x_dev);
+/* DagmaLinear('l2', trek_reg=PST(seq="inv", mode="opt")).minimize / fit for a batch of problems;
+ * src/dagma/linear.py:165-333, 441-457 with the trek term of :224-276, src/notreks/notreks.py:500-507, 599-619:
+ *   Gobj += w_b * 2 W o GT^T,  GT = X Gt X,  X = ((1 + eps_inv) I - W o W)^{-1},  obj += w_b * pst(W).
+ * Pairs of problem b: pairs_dev[pair_off_dev[b] .. pair_off_dev[b + 1]) as (i, j) int32 pairs, 0 <= i, j < d, duplicates
+ * accumulate; pair_off_dev [batch + 1] with pair_off_dev[0] = 0; pairs_dev 8-byte aligned and non-NULL (also when
+ * there are no pairs).  trek_weight_dev [batch] = w_b.  A problem without pairs has no trek term.  agg (DAGMA_PST_*)
+ * and eps_inv are shared by the batch.  1 <= d <= DAGMA_SMALL_MAX_D; args->ckpt_diag_dev must be NULL.  One CTA per
+ * problem (one per SM), pulled from the work queue.                                                              */
+#define DAGMA_PST_MEAN 0
+#define DAGMA_PST_SUM 1
+#define DAGMA_PST_MAX 2
+#define DAGMA_PST_LSE 3
+int dagma_linear_fit_small_pst_f64(dagma_stream_t stream, const dagma_small_fit_args* args,
+                                   const int32_t* pair_off_dev, const int32_t* pairs_dev,
+                                   const double* trek_weight_dev, int agg, double eps_inv);
 /* launch geometry chosen for (d): CTAs, threads, dynamic shared memory bytes */
 int dagma_linear_fit_small_geometry(int d, int batch, int* ctas, int* threads, size_t* smem_bytes);
 

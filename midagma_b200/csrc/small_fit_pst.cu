@@ -1,0 +1,604 @@
+// Batched DagmaLinear('l2', trek_reg=PST(seq="inv", mode="opt")).minimize / fit for 1 <= d <= 64: one CTA per
+// problem runs the whole schedule (stages, retries, back-tracking, checkpoints) -- the trek-regularised sibling of
+// fit_small_dmma_kernel (small_fit_dmma.cu) and fit_small_logistic_kernel (small_fit_logistic.cu), with the same
+// contract (dagma_small_fit_args) and the same reference semantics (src/dagma/linear.py:165-333 inner loop, :441-457
+// stage loop; quirks Q1-Q7 of SURVEY.md 8), plus the PST term of src/dagma/linear.py:224-276 and
+// src/notreks/notreks.py:500-507, 599-619 with the closed-form adjoint of _pst.py:
+//
+//   X   = ((1 + eps) I - W o W)^{-1}                (a second block Gauss-Jordan sweep, no domain check)
+//   v_p = H[i_p, j_p],  H = X^T X                   (only the m pair values, each a dot product of two columns of X)
+//   G_S = G_H + G_H^T                               (pair weights: mean 1/m, sum 1, max ties share, lse softmax(v))
+//   GT^T = X^T (X G_S) X^T                          (= (X Gt X)^T with Gt = G_F^T, G_F = X G_S: three DMMA products)
+//   Gobj += weight * 2 W o GT^T;  obj += weight * pst(W) at the checkpoints
+//
+// Mapping (256 threads, ONE CTA per SM -- X, G_S and the product buffer take 102 KB of shared memory next to the 87 KB
+// of the l2 sweep; problems pulled from an atomic work queue, no grid barriers):
+//   * sweep 1 inverts M^T = sI - (W o W)^T with the score GEMM cov (I - W) as filler work, as in the l2 kernel; the
+//     gradient without the trek term and the feasibility flag are formed right after it, the former parked in tensor
+//     memory next to the Adam moments, so the registers are free for sweep 2;
+//   * pair weights are scattered into G_S with shared-memory atomics.  Every contribution to one entry comes from pairs
+//     with the same unordered key {i, j}, whose values are bit-identical (each computed in the order of (min, max)),
+//     so all addends of one entry are equal and their sum does not depend on the order the atomics land in.  The
+//     normalisation (1/m, 1/ties, 1/sum exp) is applied to GT^T as one scalar; for mean / sum G_S is built once per
+//     problem and the pair values are only needed at the checkpoints.
+#include "common.cuh"
+#define DAGMA_SWEEP_JIT_ROWS 1        // the score filler's accumulators need the registers of the row fragments
+#include "small_dmma.cuh"
+#include "fit_step.cuh"
+#include "../../include/dagma_b200.h"
+
+namespace dagma {
+
+constexpr int PS_TMEM_COLS = 256;         // per thread: m, v (64 columns) and the gradient without the trek term (32)
+
+struct PstSmem {                          // offsets in doubles; the sweep's buffers keep the offsets of DmmaSmem
+    static constexpr int X = DmmaSmem::total;                 // [64][68] X = ((1 + eps) I - W o W)^{-1}
+    static constexpr int GS = X + DM_DP * DM_LD;              // [64][68] G_H + G_H^T, un-normalised
+    static constexpr int P = GS + DM_DP * DM_LD;              // [64][68] G_F, then G_F X^T
+    static constexpr int total = P + DM_DP * DM_LD;
+    static constexpr size_t bytes = (size_t)total * sizeof(double);
+};
+static_assert(PstSmem::X % 2 == 0, "16-byte alignment of vector accesses");
+
+// acc = A B over k < 4 nk on DMMA.8x8x4, accumulator ownership of DmmaPos; A(r, k) = TA ? A[k][r] : A[r][k] and
+// B(k, c) = TB ? B[c][k] : B[k][c], both [64][DM_LD].  Warps whose tiles lie outside d x d get zeros.
+template <bool TA, bool TB>
+__device__ __forceinline__ void pst_product(double (&acc)[2][4][2], const DmmaPos& ps, const double* A, const double* B,
+                                            int d) {
+#pragma unroll
+    for (int ti = 0; ti < 2; ++ti)
+#pragma unroll
+        for (int tj = 0; tj < 4; ++tj) acc[ti][tj][0] = acc[ti][tj][1] = 0.0;
+    if (16 * ps.wr >= d || 32 * ps.wc >= d) return;
+    const int nk = (d + 3) >> 2;
+#pragma unroll 2
+    for (int kb = 0; kb < nk; ++kb) {
+        const int k = 4 * kb + ps.qc;
+        double a[2], b[4];
+#pragma unroll
+        for (int ti = 0; ti < 2; ++ti) {
+            const int r = ps.row(ti);
+            a[ti] = TA ? A[k * DM_LD + r] : A[r * DM_LD + k];
+        }
+#pragma unroll
+        for (int tj = 0; tj < 4; ++tj) {
+            const int c = 32 * ps.wc + 8 * tj + ps.qr;
+            b[tj] = TB ? B[c * DM_LD + k] : B[k * DM_LD + c];
+        }
+#pragma unroll
+        for (int ti = 0; ti < 2; ++ti)
+#pragma unroll
+            for (int tj = 0; tj < 4; ++tj) dmma(acc[ti][tj][0], acc[ti][tj][1], a[ti], b[tj]);
+    }
+}
+
+__device__ __forceinline__ void store_tiles(double* dst, const double (&acc)[2][4][2], const DmmaPos& ps) {
+#pragma unroll
+    for (int ti = 0; ti < 2; ++ti)
+#pragma unroll
+        for (int tj = 0; tj < 4; ++tj)
+            *reinterpret_cast<double2*>(dst + ps.row(ti) * DM_LD + ps.col(tj)) = make_double2(acc[ti][tj][0], acc[ti][tj][1]);
+}
+
+// H[i][j] = sum_k X[k][i] X[k][j] in the order of the unordered pair: (i, j) and (j, i) give the same bits
+__device__ __forceinline__ double pair_value(const double* Xs, int d, int i, int j) {
+    const int lo = min(i, j), hi = max(i, j);
+    double v = 0.0;
+#pragma unroll 4
+    for (int k = 0; k < d; ++k) v = fma(Xs[k * DM_LD + lo], Xs[k * DM_LD + hi], v);
+    return v;
+}
+
+__device__ __forceinline__ void scatter_pair(double* GS, int i, int j, double g) {
+    atomicAdd(GS + i * DM_LD + j, g);       // G_H
+    atomicAdd(GS + j * DM_LD + i, g);       // G_H^T
+}
+
+__global__ void __launch_bounds__(DM_NT, 1) fit_small_pst_kernel(const dagma_small_fit_args P,
+                                                                  const int32_t* __restrict__ pair_off,
+                                                                  const int32_t* __restrict__ pairs,
+                                                                  const double* __restrict__ trek_weight, int agg,
+                                                                  double eps_inv) {
+    using S = DmmaSmem;
+    constexpr int NT = DM_NT, LD = DM_LD;
+    extern __shared__ __align__(16) double smem[];
+    double* ncov = smem + S::ncov;
+    double* Ws = smem + S::W;
+    double* pinfo = smem + S::pinfo;
+    double* red = smem + S::red;
+    double* Xs = smem + PstSmem::X;
+    double* GS = smem + PstSmem::GS;
+    double* Ps = smem + PstSmem::P;
+    __shared__ unsigned s_prob;
+    __shared__ uint32_t s_tmem;
+    // Adam bias correction, kept by one lane (see fit_small_dmma_kernel)
+    __shared__ double s_pow[4];
+    __shared__ double s_pow_next[4];
+    __shared__ double s_bias[2][2];
+
+    const int tid = threadIdx.x;
+    const DmmaPos ps(tid);
+    const int d = P.d;
+    const int np = 4 * ((d + 3) >> 2);
+    const size_t dd = (size_t)d * d;
+    const bool pair_agg = agg == DAGMA_PST_MAX || agg == DAGMA_PST_LSE;   // G_S depends on the pair values
+
+    SweepSync sy{smem_u32(smem + S::mbar), 0u};
+    if (tid == 0) mbar_init(sy.bar, NT / 32);
+
+    if (ps.warp == 0) tmem_alloc<PS_TMEM_COLS>(smem_u32(&s_tmem));
+    tmem_fence_before();
+    __syncthreads();
+    tmem_fence_after();
+    const uint32_t tmem_base = s_tmem;
+    // columns of a thread: [m(ti=0) 16 | v(ti=0) 16 | m(ti=1) 16 | v(ti=1) 16 | Gobj0(ti=0) 16 | Gobj0(ti=1) 16]
+    const uint32_t tm = tmem_base + ((uint32_t)(32 * (ps.warp & 3)) << 16) + (uint32_t)((ps.warp >> 2) * 96);
+    const uint32_t tg = tm + 64;
+
+    unsigned excbits = 0, incbits = 0;
+#pragma unroll
+    for (int ti = 0; ti < 2; ++ti)
+#pragma unroll
+        for (int tj = 0; tj < 4; ++tj)
+#pragma unroll
+            for (int e = 0; e < 2; ++e) {
+                const int r = ps.row(ti), c = ps.col(tj) + e;
+                if (r < d && c < d) {
+                    if (P.mask_exc_dev && P.mask_exc_dev[r * d + c]) excbits |= 1u << (ti * 8 + tj * 2 + e);
+                    if (P.mask_inc_dev && P.mask_inc_dev[r * d + c]) incbits |= 1u << (ti * 8 + tj * 2 + e);
+                }
+            }
+
+    for (;;) {
+        if (tid == 0) s_prob = atomicAdd(P.work_counter_dev, 1u);
+        __syncthreads();
+        const unsigned b = s_prob;
+        __syncthreads();
+        if (b >= (unsigned)P.batch) break;
+
+        const double* cov_g = P.cov_dev + (size_t)b * dd;
+        double* W_g = P.w_dev + (size_t)b * dd;
+        const double lambda1 = P.lambda1_dev[b];
+        const int p0 = pair_off[b];
+        const int m = pair_off[b + 1] - p0;
+        const int2* pr = reinterpret_cast<const int2*>(pairs) + p0;
+        const double weight = trek_weight[b];
+
+        for (int idx = tid; idx < DM_DP * DM_DP; idx += NT) {
+            const int r = idx >> 6, c = idx & 63;
+            const bool in = (r < d) && (c < d);
+            ncov[r * LD + c] = in ? -cov_g[r * d + c] : 0.0;
+            Ws[r * LD + c] = in ? W_g[r * d + c] : 0.0;
+        }
+        for (int e = tid; e < DM_DP * LD; e += NT) GS[e] = 0.0;
+        __syncthreads();
+        if (m > 0 && !pair_agg) {                       // mean / sum: G_S counts the pairs, fixed for the problem
+            for (int p = tid; p < m; p += NT) {
+                const int2 ij = pr[p];
+                scatter_pair(GS, ij.x, ij.y, 1.0);
+            }
+        }
+        __syncthreads();
+
+        double a[2][4][2], g[2][4][2];
+        int status = 0;
+        int n_ckpt = 0;
+
+        int stage = 0;
+        bool final_phase = (P.n_stages == 0);
+        double mu = 0, s_cur = 1, lr = 0, lr_adam = P.lr, obj_prev = 1e16;
+        double last_obj = 0, last_score = 0, last_h = 0;
+        int iters_max = 0, it = 0, retries = 0, backtracks = 0;
+        bool in_backtrack = false;
+
+        auto start_attempt = [&]() {
+            it = 0;
+            lr = lr_adam;
+            obj_prev = 1e16;
+            in_backtrack = false;
+            backtracks = 0;
+            if (tid == DM_NT - 32) { s_pow[0] = 1.0; s_pow[1] = 0.0; s_pow[2] = 1.0; s_pow[3] = 0.0; }
+            const double z[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+#pragma unroll
+            for (int q = 0; q < 4; ++q) tmem_st8(tm + 16 * q, z);
+            tmem_wait_st();
+        };
+        auto start_stage = [&]() {
+            mu = P.mu[stage];
+            s_cur = P.s[stage];
+            iters_max = P.iters[stage];
+            lr_adam = P.lr;
+            retries = 0;
+            start_attempt();
+        };
+        auto write_W = [&]() {
+            __syncthreads();
+            for (int idx = tid; idx < d * d; idx += NT) {
+                const int r = idx / d, c = idx - r * d;
+                W_g[idx] = Ws[r * LD + c];
+            }
+        };
+        auto read_W = [&]() {
+            __syncthreads();
+            for (int idx = tid; idx < d * d; idx += NT) {
+                const int r = idx / d, c = idx - r * d;
+                Ws[r * LD + c] = W_g[idx];
+            }
+            __syncthreads();
+        };
+        auto write_stage_stats = [&]() {
+            if (tid == 0 && P.stage_stats_dev) {
+                double* st = P.stage_stats_dev + ((size_t)b * P.n_stages + stage) * 8;
+                st[0] = (double)it;
+                st[1] = lr;
+                st[2] = s_cur;
+                st[3] = last_obj;
+                st[4] = last_score;
+                st[5] = last_h;
+                st[6] = (double)retries;
+                st[7] = (double)backtracks;
+            }
+        };
+        // Ws += scale * dir(m, v, it): the previous Adam direction rebuilt from the moments
+        auto apply_dir = [&](double scale) {
+            const double c1 = s_bias[it & 1][0] * (1.0 - P.beta1), c2 = s_bias[it & 1][1] * (1.0 - P.beta2);
+#pragma unroll
+            for (int ti = 0; ti < 2; ++ti) {
+                TmemLoad8 lm, lv;
+                lm.issue(tm + 32 * ti);
+                lv.issue(tm + 32 * ti + 16);
+                lm.finish();
+                lv.finish();
+                double* wp = Ws + ps.row(ti) * LD;
+#pragma unroll
+                for (int tj = 0; tj < 4; ++tj) {
+                    double2 w = *reinterpret_cast<double2*>(wp + ps.col(tj));
+                    const double d0 = fast_div(lm.get(2 * tj) * c1, fast_sqrt_nonneg(lv.get(2 * tj) * c2) + 1e-8);
+                    const double d1 = fast_div(lm.get(2 * tj + 1) * c1, fast_sqrt_nonneg(lv.get(2 * tj + 1) * c2) + 1e-8);
+                    w.x = __dadd_rn(w.x, __dmul_rn(scale, d0));
+                    w.y = __dadd_rn(w.y, __dmul_rn(scale, d1));
+                    *reinterpret_cast<double2*>(wp + ps.col(tj)) = w;
+                }
+            }
+            __syncthreads();
+        };
+
+        if (!final_phase) start_stage();
+
+        for (;;) {
+            const double s_use = final_phase ? 1.0 : s_cur;
+            const bool at_ckpt = !final_phase && !in_backtrack && it >= 1 &&
+                                 (it % P.checkpoint == 0 || it == iters_max);
+            // ================= sweep 1: M^{-T}, with g = cov (I - W) as filler work =================
+#pragma unroll
+            for (int ti = 0; ti < 2; ++ti) {
+                const int r = ps.row(ti);
+#pragma unroll
+                for (int tj = 0; tj < 4; ++tj) {
+                    const int c = ps.col(tj);
+                    const double w0 = Ws[c * LD + r], w1 = Ws[(c + 1) * LD + r];     // W^T
+                    const double dg = (r < d) ? s_use : 1.0;
+                    a[ti][tj][0] = ((r == c) ? dg : 0.0) - w0 * w0;
+                    a[ti][tj][1] = ((r == c + 1) ? dg : 0.0) - w1 * w1;
+                    const double2 nc = *reinterpret_cast<const double2*>(ncov + r * LD + c);
+                    g[ti][tj][0] = -nc.x;
+                    g[ti][tj][1] = -nc.y;
+                }
+            }
+            if (tid == DM_NT - 32 && !final_phase) {      // bias factors of iteration it + 1
+                DD q1{s_pow[0], s_pow[1]}, q2{s_pow[2], s_pow[3]};
+                q1.mul(P.beta1);
+                q2.mul(P.beta2);
+                s_pow_next[0] = q1.hi; s_pow_next[1] = q1.lo; s_pow_next[2] = q2.hi; s_pow_next[3] = q2.lo;
+                s_bias[(it + 1) & 1][0] = fast_rcp(q1.one_minus());
+                s_bias[(it + 1) & 1][1] = fast_rcp(q2.one_minus());
+            }
+            {
+                ScoreFill fill{g, ps, smem, 0, (d + 3) >> 2};
+                dmma_sweep(a, ps, smem, d, sy, fill);
+#pragma unroll 1
+                while (fill.more()) fill.unit();
+            }
+            // now: a = M^{-T},  g = cov (I - W),  pinfo[0..np) = pivots
+
+            // ================= objective without the trek term (checkpoint / final) =================
+            double score = 0.0, h = 0.0, l1 = 0.0;
+            if (at_ckpt || final_phase) {
+                double sc = 0.0, ld = 0.0;
+#pragma unroll
+                for (int ti = 0; ti < 2; ++ti) {
+                    const int r = ps.row(ti);
+#pragma unroll
+                    for (int tj = 0; tj < 4; ++tj) {
+                        const int c = ps.col(tj);
+                        const double2 w = *reinterpret_cast<const double2*>(Ws + r * LD + c);
+                        const double dif0 = ((r == c && r < d) ? 1.0 : 0.0) - w.x;
+                        const double dif1 = ((r == c + 1 && r < d) ? 1.0 : 0.0) - w.y;
+                        sc = fma(dif0, g[ti][tj][0], sc);
+                        sc = fma(dif1, g[ti][tj][1], sc);
+                        l1 += fabs(w.x) + fabs(w.y);
+                    }
+                }
+                if (tid < np) ld = (double)((tid & 3) - 2) * log(fabs(pinfo[tid]));
+                block_sum3<NT>(sc, l1, ld, red, tid);
+                score = 0.5 * sc;
+                h = -ld + (double)d * log(s_use);
+                if (final_phase) {
+                    if (tid == 0 && P.final_dev) {
+                        P.final_dev[2 * (size_t)b] = h;
+                        P.final_dev[2 * (size_t)b + 1] = score;
+                    }
+                    break;
+                }
+            }
+
+            // ================= feasibility of iteration it + 1 (sweep 2 overwrites pinfo) =================
+            bool bad = false;
+            if (tid < np) bad = !(pinfo[tid] > 0.0);
+#pragma unroll
+            for (int ti = 0; ti < 2; ++ti)
+#pragma unroll
+                for (int tj = 0; tj < 4; ++tj)
+                    bad |= below_minus_1e16(a[ti][tj][0]) | below_minus_1e16(a[ti][tj][1]);
+            bad = __syncthreads_or(bad);
+
+            if (!bad) {
+                // Gobj without the trek term = -mu cov (I - W) + mu l1 sign(W) + 2 W o (M^{-T} + 1e-16) (+ include
+                // mask), linear.py:248, parked in tensor memory while sweep 2 needs the registers
+                const double l1c = mu * lambda1, incc = -2.0 * mu * lambda1, nmu = -mu;
+#pragma unroll
+                for (int ti = 0; ti < 2; ++ti) {
+                    const double* wp = Ws + ps.row(ti) * LD;
+                    double go[8];
+#pragma unroll
+                    for (int q = 0; q < 8; ++q) {
+                        const double w = wp[ps.col(q >> 1) + (q & 1)];
+                        go[q] = fma(nmu, g[ti][q >> 1][q & 1], signed_const(w, l1c));
+                        go[q] = fma(twice(w), a[ti][q >> 1][q & 1] + 1e-16, go[q]);
+                        if (incbits >> (ti * 8 + q) & 1u) go[q] += signed_const(w, incc);
+                    }
+                    tmem_st8(tg + 16 * ti, go);
+                }
+                tmem_wait_st();
+            }
+
+            // ================= PST inv at the current W =================
+            double tval = 0.0, tscale = 0.0;
+            double t[2][4][2];
+            const bool trek = m > 0 && (at_ckpt || !bad);
+            if (trek) {
+                const double dgx = 1.0 + eps_inv;
+#pragma unroll
+                for (int ti = 0; ti < 2; ++ti) {
+                    const int r = ps.row(ti);
+#pragma unroll
+                    for (int tj = 0; tj < 4; ++tj) {
+                        const int c = ps.col(tj);
+                        const double2 w = *reinterpret_cast<const double2*>(Ws + r * LD + c);
+                        const double dg = (r < d) ? dgx : 1.0;
+                        a[ti][tj][0] = ((r == c) ? dg : 0.0) - w.x * w.x;
+                        a[ti][tj][1] = ((r == c + 1) ? dg : 0.0) - w.y * w.y;
+                    }
+                }
+                dmma_sweep(a, ps, smem, d, sy);
+                store_tiles(Xs, a, ps);
+                if (pair_agg)
+                    for (int idx = tid; idx < d * d; idx += NT) GS[(idx / d) * LD + idx % d] = 0.0;
+                __syncthreads();
+                // pair values -> value and the un-normalised pair weights; tscale = weight x normalisation
+                if (!pair_agg) {
+                    if (at_ckpt) {
+                        double sv = 0.0, z1 = 0.0, z2 = 0.0;
+                        for (int p = tid; p < m; p += NT) {
+                            const int2 ij = pr[p];
+                            sv += pair_value(Xs, d, ij.x, ij.y);
+                        }
+                        block_sum3<NT>(sv, z1, z2, red, tid);
+                        tval = (agg == DAGMA_PST_MEAN) ? sv / (double)m : sv;
+                    }
+                    tscale = (agg == DAGMA_PST_MEAN) ? weight / (double)m : weight;
+                } else {
+                    double mx = -INFINITY;
+                    for (int p = tid; p < m; p += NT) {
+                        const int2 ij = pr[p];
+                        mx = fmax(mx, pair_value(Xs, d, ij.x, ij.y));
+                    }
+                    mx = block_max<NT>(mx, red, tid);
+                    double se = 0.0, z1 = 0.0, z2 = 0.0;
+                    for (int p = tid; p < m; p += NT) {
+                        const int2 ij = pr[p];
+                        const double v = pair_value(Xs, d, ij.x, ij.y);
+                        if (agg == DAGMA_PST_MAX) {
+                            if (v == mx) {                  // torch shares the gradient of max() between ties
+                                se += 1.0;
+                                scatter_pair(GS, ij.x, ij.y, 1.0);
+                            }
+                        } else {
+                            const double e = exp(v - mx);
+                            se += e;
+                            scatter_pair(GS, ij.x, ij.y, e);
+                        }
+                    }
+                    block_sum3<NT>(se, z1, z2, red, tid);   // (its barriers also publish the scatter)
+                    tval = (agg == DAGMA_PST_MAX) ? mx : mx + log(se);
+                    tscale = weight / se;
+                }
+                // GT^T = X^T (X G_S) X^T
+                pst_product<false, false>(t, ps, Xs, GS, d);       // G_F = X G_S
+                store_tiles(Ps, t, ps);
+                __syncthreads();
+                pst_product<false, true>(t, ps, Ps, Xs, d);        // U = G_F X^T
+                __syncthreads();
+                store_tiles(Ps, t, ps);
+                __syncthreads();
+                pst_product<true, false>(t, ps, Xs, Ps, d);        // GT^T = X^T U
+            }
+
+            if (at_ckpt) {
+                const double obj = mu * (score + lambda1 * l1) + h + weight * tval;
+                last_obj = obj;
+                last_score = score;
+                last_h = h;
+                if (tid == 0 && P.ckpt_log_dev && n_ckpt < P.ckpt_log_cap) {
+                    double* row = P.ckpt_log_dev + ((size_t)b * P.ckpt_log_cap + n_ckpt) * 6;
+                    row[0] = stage; row[1] = it; row[2] = obj; row[3] = score; row[4] = h; row[5] = lr;
+                }
+                ++n_ckpt;
+                const bool converged = fabs((obj_prev - obj) / obj_prev) <= P.tol;
+                obj_prev = obj;
+                if (converged || it == iters_max) goto stage_done;
+            } else if (!in_backtrack && it == iters_max) {
+                goto stage_done;   // only reachable for iters_max == 0
+            }
+
+            if (bad) {
+                if (it == 0 || s_cur <= 0.9) {            // linear.py:231-233
+                    if (P.retry_on_fail) {
+                        if (++retries > 64) {
+                            status |= DAGMA_ST_RETRY_LIMIT;
+                            --retries;
+                            read_W();
+                            write_stage_stats();
+                            if (!P.final_dev) goto problem_done;
+                            final_phase = true;
+                            continue;
+                        }
+                        lr_adam *= 0.5;                    // linear.py:450-451
+                        s_cur += 0.1;
+                        read_W();
+                        start_attempt();
+                        continue;
+                    }
+                    status |= DAGMA_ST_OUT_OF_DOMAIN;
+                    write_W();
+                    write_stage_stats();
+                    goto problem_done;
+                }
+                apply_dir(lr);                             // W += lr * grad   :235
+                lr *= 0.5;                                 //                  :236
+                if (lr <= 1e-16) {                         //                  :237-238
+                    status |= DAGMA_ST_LR_UNDERFLOW;
+                    goto stage_done;
+                }
+                apply_dir(-lr);                            // W -= lr * grad   :239
+                ++backtracks;
+                in_backtrack = true;
+                continue;                                  // re-invert        :240
+            }
+            in_backtrack = false;
+
+            {
+                // ================= Adam step (iteration it + 1) =================
+                ++it;
+                const double k1 = s_bias[it & 1][0] * (1.0 - P.beta1), k2 = s_bias[it & 1][1] * (1.0 - P.beta2);
+                if (tid == DM_NT - 32) {
+                    s_pow[0] = s_pow_next[0]; s_pow[1] = s_pow_next[1]; s_pow[2] = s_pow_next[2]; s_pow[3] = s_pow_next[3];
+                }
+#pragma unroll
+                for (int ti = 0; ti < 2; ++ti) {
+                    TmemLoad8 lm, lv, lg;
+                    lg.issue(tg + 16 * ti);
+                    lm.issue(tm + 32 * ti);
+                    lv.issue(tm + 32 * ti + 16);
+                    double* wp = Ws + ps.row(ti) * LD;
+                    double w[8], go[8], mn[8], vn[8];
+#pragma unroll
+                    for (int tj = 0; tj < 4; ++tj) {
+                        const double2 v2 = *reinterpret_cast<const double2*>(wp + ps.col(tj));
+                        w[2 * tj] = v2.x;
+                        w[2 * tj + 1] = v2.y;
+                    }
+                    lg.finish();
+#pragma unroll
+                    for (int q = 0; q < 8; ++q) go[q] = lg.get(q);
+                    if (trek) {                            // + weight * 2 W o GT^T   (linear.py:251-258)
+#pragma unroll
+                        for (int q = 0; q < 8; ++q) go[q] = fma(twice(w[q]), tscale * t[ti][q >> 1][q & 1], go[q]);
+                    }
+                    lm.finish();
+                    lv.finish();
+#pragma unroll
+                    for (int q = 0; q < 8; ++q) {
+                        mn[q] = lm.get(q);
+                        vn[q] = lv.get(q);
+                    }
+#pragma unroll
+                    for (int q0 = 0; q0 < 8; q0 += DAGMA_ADAM_GROUP)
+                        adam_entries<DAGMA_ADAM_GROUP>(w + q0, go + q0, mn + q0, vn + q0, P.beta1, P.beta2, k1, k2, lr);
+                    tmem_st8(tm + 32 * ti, mn);
+                    tmem_st8(tm + 32 * ti + 16, vn);
+#pragma unroll
+                    for (int tj = 0; tj < 4; ++tj) {
+                        double2 v2 = make_double2(w[2 * tj], w[2 * tj + 1]);
+                        if (excbits >> (ti * 8 + 2 * tj) & 1u) v2.x = 0.0;
+                        if (excbits >> (ti * 8 + 2 * tj + 1) & 1u) v2.y = 0.0;
+                        *reinterpret_cast<double2*>(wp + ps.col(tj)) = v2;
+                    }
+                }
+                tmem_wait_st();
+                __syncthreads();
+                continue;
+            }
+
+        stage_done:
+            write_stage_stats();
+            write_W();
+            ++stage;
+            if (stage < P.n_stages) {
+                start_stage();
+                __syncthreads();
+                continue;
+            }
+            if (!P.final_dev) goto problem_done;
+            final_phase = true;
+            __syncthreads();
+        }
+    problem_done:
+        if (tid == 0) {
+            if (P.status_dev) P.status_dev[b] = status;
+            if (P.ckpt_count_dev) P.ckpt_count_dev[b] = n_ckpt < P.ckpt_log_cap ? n_ckpt : P.ckpt_log_cap;
+        }
+        __syncthreads();
+    }
+
+    tmem_fence_before();
+    __syncthreads();
+    if (ps.warp == 0) tmem_free<PS_TMEM_COLS>(tmem_base);
+}
+
+}  // namespace dagma
+
+using namespace dagma;
+
+extern "C" int dagma_linear_fit_small_pst_f64(dagma_stream_t stream_, const dagma_small_fit_args* args,
+                                              const int32_t* pair_off_dev, const int32_t* pairs_dev,
+                                              const double* trek_weight_dev, int agg, double eps_inv) {
+    DAGMA_REQUIRE(args != nullptr, "null args");
+    const dagma_small_fit_args& a = *args;
+    DAGMA_REQUIRE(a.batch >= 1, "batch must be positive");
+    DAGMA_REQUIRE(a.d >= 1 && a.d <= DAGMA_SMALL_MAX_D, "d out of range for the on-chip PST fit");
+    DAGMA_REQUIRE(a.n_stages >= 0 && a.n_stages <= DAGMA_MAX_STAGES, "too many stages");
+    DAGMA_REQUIRE(a.checkpoint >= 1, "checkpoint must be >= 1");
+    DAGMA_REQUIRE(a.cov_dev && a.w_dev && a.lambda1_dev && a.work_counter_dev, "null device pointer");
+    DAGMA_REQUIRE(pair_off_dev && pairs_dev && trek_weight_dev, "null pair / weight pointer");
+    DAGMA_REQUIRE(agg >= DAGMA_PST_MEAN && agg <= DAGMA_PST_LSE, "agg must be one of DAGMA_PST_MEAN .. DAGMA_PST_LSE");
+    DAGMA_REQUIRE(eps_inv >= 0.0 && eps_inv < 1e300, "eps_inv must be finite and >= 0");
+    DAGMA_REQUIRE(a.ckpt_diag_dev == nullptr, "the PST fit writes no telemetry rows (ckpt_diag_dev must be NULL)");
+    DAGMA_REQUIRE(((uintptr_t)pairs_dev & 7u) == 0, "pairs_dev must be 8-byte aligned");
+    cudaStream_t stream = (cudaStream_t)stream_;
+    int dev = 0, sms = 0;
+    DAGMA_CUDA_OK(cudaGetDevice(&dev));
+    DAGMA_CUDA_OK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    DAGMA_CUDA_OK(cudaFuncSetAttribute(fit_small_pst_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                       (int)PstSmem::bytes));
+    DAGMA_CUDA_OK(cudaFuncSetAttribute(fit_small_pst_kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
+                                       cudaSharedmemCarveoutMaxShared));
+    // one CTA per SM: 189 KB of shared memory; 256 TMEM columns of the 512 of an SM
+    long ctas = sms;
+    if (ctas > a.batch) ctas = a.batch;
+    DAGMA_CUDA_OK(cudaMemsetAsync(a.work_counter_dev, 0, sizeof(uint32_t), stream));
+    fit_small_pst_kernel<<<(int)ctas, DM_NT, PstSmem::bytes, stream>>>(a, pair_off_dev, pairs_dev, trek_weight_dev, agg,
+                                                                        eps_inv);
+    DAGMA_CUDA_OK(cudaGetLastError());
+    return 0;
+}

@@ -58,9 +58,10 @@ class SmallFitResult(typing.NamedTuple):
 
 def _run_small(cov: torch.Tensor, W: torch.Tensor, lambda1: torch.Tensor, mus, ss, iters, *, lr, tol,
                beta1, beta2, checkpoint, retry, mask_exc=None, mask_inc=None, ckpt_log_cap=0,
-               want_final=True, want_diag=False, X=None) -> SmallFitResult:
+               want_final=True, want_diag=False, X=None, pst=None) -> SmallFitResult:
     """Launch ``dagma_linear_fit_small_f64`` on device tensors (W is updated in place).  With ``X`` ([batch, n, d]
-    device tensor; ``cov`` = its un-centred X^T X / n) the logistic loss: ``dagma_linear_fit_small_logistic_f64``."""
+    device tensor; ``cov`` = its un-centred X^T X / n) the logistic loss: ``dagma_linear_fit_small_logistic_f64``.
+    With ``pst`` (a ``_PstBatch``) the l2 loss plus the PST ``inv`` term: ``dagma_linear_fit_small_pst_f64``."""
     _lib.require_device()
     lib = _lib.load()
     batch, d, _ = cov.shape
@@ -68,7 +69,7 @@ def _run_small(cov: torch.Tensor, W: torch.Tensor, lambda1: torch.Tensor, mus, s
     if T > _lib.MAX_STAGES:
         return _run_small_chunked(cov, W, lambda1, mus, ss, iters, lr=lr, tol=tol, beta1=beta1, beta2=beta2,
                                   checkpoint=checkpoint, retry=retry, mask_exc=mask_exc, mask_inc=mask_inc,
-                                  ckpt_log_cap=ckpt_log_cap, want_final=want_final, want_diag=want_diag, X=X)
+                                  ckpt_log_cap=ckpt_log_cap, want_final=want_final, want_diag=want_diag, X=X, pst=pst)
     assert cov.is_cuda and W.is_cuda and cov.dtype == torch.float64 and W.dtype == torch.float64
     assert cov.is_contiguous() and W.is_contiguous() and lambda1.is_contiguous()
     dev = cov.device
@@ -97,7 +98,12 @@ def _run_small(cov: torch.Tensor, W: torch.Tensor, lambda1: torch.Tensor, mus, s
     a.ckpt_log = log.data_ptr() if log is not None else None
     a.ckpt_count = cnt.data_ptr() if cnt is not None else None
     a.work_counter = counter.data_ptr()
-    if X is None:
+    if pst is not None:
+        assert X is None and pst.pair_off.shape[0] == batch + 1
+        _lib.check(lib.dagma_linear_fit_small_pst_f64(_lib.stream_ptr(), C.byref(a), pst.pair_off.data_ptr(),
+                                                      pst.pairs.data_ptr(), pst.weight.data_ptr(), pst.agg,
+                                                      pst.eps_inv), "dagma_linear_fit_small_pst_f64")
+    elif X is None:
         _lib.check(lib.dagma_linear_fit_small_f64(_lib.stream_ptr(), C.byref(a)), "dagma_linear_fit_small_f64")
     else:
         assert X.is_cuda and X.dtype == torch.float64 and X.is_contiguous() and X.shape[0] == batch and X.shape[2] == d
@@ -232,19 +238,81 @@ def _batch_masks(exclude_edges, include_edges, d, device):
     return out
 
 
+_PST_AGGS = {"mean": 0, "sum": 1, "max": 2, "lse": 3}       # DAGMA_PST_* of include/dagma_b200.h
+
+
+class _PstBatch(typing.NamedTuple):
+    """Pair sets of an on-chip PST ``inv`` batch in the CSR form of ``dagma_linear_fit_small_pst_f64``."""
+    pair_off: torch.Tensor      # [batch + 1] int32
+    pairs: torch.Tensor         # [max(total, 1), 2] int32
+    weight: torch.Tensor        # [batch] float64
+    agg: int
+    eps_inv: float
+
+
+def _trek_batch(trek_reg, batch: int, d: int, loss_type: str, who: str):
+    """``trek_reg`` of a batched call, checked without a device: one regulariser for the whole batch or a sequence with
+    one regulariser (or None) per problem, each validated as ``DagmaLinear(trek_reg=...)`` validates it.
+
+    Returns None when no problem carries a term that changes W (None, disabled, empty ``I``, mode "log": the reference
+    only logs such a value, linear.py:122-133, 251-258).  Otherwise ``(regs, onchip)``: ``regs`` one regulariser per
+    problem; ``onchip`` the host arrays of the PST ``inv`` kernel -- l2, d <= 64, every term PST ``inv`` with one
+    ``agg`` and ``eps_inv`` -- or None when the problems run one after the other as ``DagmaLinear(trek_reg=regs[b])``."""
+    if trek_reg is None:
+        return None
+    regs = list(trek_reg) if isinstance(trek_reg, (list, tuple)) else [trek_reg] * batch
+    if len(regs) != batch:
+        raise ValueError(f"{who}: trek_reg has {len(regs)} entries for a batch of {batch} problems")
+    plans = [_trek_plan(r) for r in regs]
+    plans = [p if p is not None and p["mode"] == "opt" else None for p in plans]
+    active = [p for p in plans if p is not None]
+    if not active:
+        return None
+    keys = {(p["kind"], p.get("seq"), p.get("agg"), p.get("eps_inv")) for p in active}
+    if loss_type != "l2" or d > _lib.SMALL_MAX_D or len(keys) != 1 or next(iter(keys))[:2] != ("pst", "inv"):
+        return regs, None
+    _, _, agg, eps_inv = keys.pop()
+    off = np.zeros(batch + 1, dtype=np.int64)
+    weight = np.zeros(batch)
+    parts = []
+    for b, p in enumerate(plans):
+        I = p["I"] if p is not None else np.zeros((0, 2), dtype=np.int64)
+        if I.size and (I.min() < -d or I.max() >= d):
+            raise IndexError(f"{who}: trek_reg of problem {b} has a pair index outside [-{d}, {d})")
+        parts.append(I % d)                       # negative indices count from the end, as H[rows, cols] does
+        off[b + 1] = off[b] + len(I)
+        weight[b] = p["weight"] if p is not None else 0.0
+    if off[-1] >= 2 ** 31:
+        raise ValueError(f"{who}: {off[-1]} trek pairs in one batch (at most 2^31 - 1)")
+    pairs = np.concatenate(parts).astype(np.int32) if off[-1] else np.zeros((1, 2), dtype=np.int32)
+    return regs, (off.astype(np.int32), pairs, weight, _PST_AGGS[agg], float(eps_inv))
+
+
+def _pst_dev(onchip, device) -> _PstBatch:
+    off, pairs, weight, agg, eps_inv = onchip
+    dev = lambda a: torch.as_tensor(np.ascontiguousarray(a)).to(device)  # noqa: E731
+    return _PstBatch(dev(off), dev(pairs), dev(weight), agg, eps_inv)
+
+
 def minimize_batch(W, cov, lambda1, mu, max_iter, s, lr, *, tol=1e-6, beta_1=0.99, beta_2=0.999,
-                   checkpoint=1000, device=None, exclude_edges=None, include_edges=None, loss_type="l2", X=None):
+                   checkpoint=1000, device=None, exclude_edges=None, include_edges=None, loss_type="l2", X=None,
+                   trek_reg=None):
     """One ``DagmaLinear(loss_type).minimize`` call (linear.py:165-333) for a batch of
     independent problems.  ``W``/``cov``: [batch, d, d] numpy arrays or torch tensors on
     host (pinned or not) or device.  ``loss_type="logistic"`` needs the data ``X`` [batch, n, d]
     (not centred, not modified); ``cov`` is then its X^T X / n and may be None (computed from X).
+    ``trek_reg``: one trek regulariser for the batch, or a sequence of one regulariser (or None)
+    per problem -- what ``DagmaLinear(loss_type, trek_reg=...)`` would carry.  l2 problems with
+    d <= 64 whose terms are all PST ``seq="inv"`` with one ``agg`` and ``eps_inv`` run in one
+    launch; other regularisers run the problems one after the other through ``DagmaLinear``.
     Like the reference, ``W`` is updated in place and returned.
     Returns ``(W, success[batch], stage_stats[batch, 1, 8])``."""
     logistic = _logistic_inputs(loss_type, X, "minimize_batch")
+    trek = _trek_batch(trek_reg, np.shape(W)[0], np.shape(W)[-1], loss_type, "minimize_batch")
     _lib.require_device()
     device = torch.device(device or "cuda")
     on_device = isinstance(W, torch.Tensor) and W.is_cuda
-    if _host_pipeline_ok(W, cov, loss_type):
+    if trek is None and _host_pipeline_ok(W, cov, loss_type):
         return _minimize_batch_host_pipelined(W, cov, lambda1, mu, max_iter, s, lr, tol=tol, beta_1=beta_1, beta_2=beta_2,
                                               checkpoint=checkpoint, device=device, exclude_edges=exclude_edges,
                                               include_edges=include_edges)
@@ -254,14 +322,15 @@ def minimize_batch(W, cov, lambda1, mu, max_iter, s, lr, *, tol=1e-6, beta_1=0.9
     batch, d, _ = covd.shape
     if Xd is not None and (Xd.shape[0] != batch or Xd.shape[2] != d):
         raise ValueError(f"minimize_batch: X {tuple(Xd.shape)} does not match W / cov [{batch}, {d}, {d}]")
-    if d > _lib.SMALL_MAX_D:
+    if d > _lib.SMALL_MAX_D or (trek is not None and trek[1] is None):
         return _minimize_batch_large(W, covd, lambda1, mu, max_iter, s, lr, tol=tol, beta_1=beta_1, beta_2=beta_2,
                                      checkpoint=checkpoint, exclude_edges=exclude_edges, include_edges=include_edges,
-                                     Xd=Xd)
+                                     Xd=Xd, treks=trek[0] if trek is not None else None)
     lam = _lam_dev(lambda1, batch, device)
     mask_exc, mask_inc = _batch_masks(exclude_edges, include_edges, d, device)
     res = _run_small(covd, Wd, lam, [mu], [s], [int(max_iter)], lr=lr, tol=tol, beta1=beta_1, beta2=beta_2,
-                     checkpoint=checkpoint, retry=False, want_final=False, mask_exc=mask_exc, mask_inc=mask_inc, X=Xd)
+                     checkpoint=checkpoint, retry=False, want_final=False, mask_exc=mask_exc, mask_inc=mask_inc, X=Xd,
+                     pst=_pst_dev(trek[1], device) if trek is not None else None)
     ok = (res.status & _lib.ST_OUT_OF_DOMAIN) == 0
     if on_device:
         if Wd is not W:
@@ -363,7 +432,7 @@ def _minimize_batch_host_pipelined(W, cov, lambda1, mu, max_iter, s, lr, *, tol,
 def fit_batch(X=None, lambda1=0.03, *, cov=None, w_threshold=0.3, T=5, mu_init=1.0, mu_factor=0.1,
               s=(1.0, .9, .8, .7, .6), warm_iter=3e4, max_iter=6e4, lr=0.0003, checkpoint=1000,
               beta_1=0.99, beta_2=0.999, tol=1e-6, device=None, return_info=False,
-              exclude_edges=None, include_edges=None, loss_type="l2"):
+              exclude_edges=None, include_edges=None, loss_type="l2", trek_reg=None):
     """``DagmaLinear(loss_type).fit`` (linear.py:335-462) for a batch of independent problems.
 
     l2: ``X``: [batch, n, d] (centred on device, the caller's array is not modified) or
@@ -372,10 +441,13 @@ def fit_batch(X=None, lambda1=0.03, *, cov=None, w_threshold=0.3, T=5, mu_init=1
     reference schedule independently (own convergence checks, retries, back-tracking);
     problems are pulled from a device-side work queue by persistent CTAs.
     ``exclude_edges`` / ``include_edges``: tuples of 2-tuples shared by the batch (linear.py:416-426).
+    ``trek_reg``: as in ``minimize_batch`` (one regulariser, or one per problem).
     Returns thresholded ``W_est`` [batch, d, d] as numpy (+ info dict)."""
     logistic = _logistic_inputs(loss_type, X, "fit_batch")
     if logistic and cov is not None:
         raise ValueError("fit_batch(loss_type='logistic') takes X only: the covariance is computed from it")
+    src = X if cov is None else cov
+    trek = _trek_batch(trek_reg, np.shape(src)[0], np.shape(src)[-1], loss_type, "fit_batch")
     _lib.require_device()
     device = torch.device(device or "cuda")
     Xd = None
@@ -391,11 +463,11 @@ def fit_batch(X=None, lambda1=0.03, *, cov=None, w_threshold=0.3, T=5, mu_init=1
     else:
         covd = _as_dev(cov, device)
     batch, d, _ = covd.shape
-    if d > _lib.SMALL_MAX_D:
+    if d > _lib.SMALL_MAX_D or (trek is not None and trek[1] is None):
         return _fit_batch_large(covd, lambda1, w_threshold=w_threshold, T=T, mu_init=mu_init, mu_factor=mu_factor, s=s,
                                 warm_iter=warm_iter, max_iter=max_iter, lr=lr, checkpoint=checkpoint, beta_1=beta_1,
                                 beta_2=beta_2, return_info=return_info, exclude_edges=exclude_edges,
-                                include_edges=include_edges, Xd=Xd)
+                                include_edges=include_edges, Xd=Xd, treks=trek[0] if trek is not None else None)
     lam = _lam_dev(lambda1, batch, device)
     T = int(T)
     ss = list(s) if isinstance(s, (list, tuple)) else T * [s]
@@ -406,7 +478,8 @@ def fit_batch(X=None, lambda1=0.03, *, cov=None, w_threshold=0.3, T=5, mu_init=1
     Wd = torch.zeros(batch, d, d, dtype=torch.float64, device=device)
     mask_exc, mask_inc = _batch_masks(exclude_edges, include_edges, d, device)
     res = _run_small(covd, Wd, lam, mus, ss[:T], iters, lr=lr, tol=tol, beta1=beta_1, beta2=beta_2,
-                     checkpoint=checkpoint, retry=True, mask_exc=mask_exc, mask_inc=mask_inc, X=Xd)
+                     checkpoint=checkpoint, retry=True, mask_exc=mask_exc, mask_inc=mask_inc, X=Xd,
+                     pst=_pst_dev(trek[1], device) if trek is not None else None)
     _warn_retry_limit(res.status)
     W_raw = res.W.cpu().numpy()
     W_est = W_raw.copy()
@@ -501,9 +574,11 @@ def _run_lanes(batch: int, d: int, solve, device, n: typing.Optional[int] = None
 
 
 def _minimize_batch_large(W, covd, lambda1, mu, max_iter, s, lr, *, tol, beta_1, beta_2, checkpoint, exclude_edges,
-                          include_edges, Xd=None):
+                          include_edges, Xd=None, treks=None):
     """``minimize_batch`` beyond the on-chip size: one ``DagmaLinear.minimize`` per problem on the multi-CTA engine, for
-    d <= 128 several problems side by side (one persistent kernel each, csrc/lin_iter.cu)."""
+    d <= 128 several problems side by side (one persistent kernel each, csrc/lin_iter.cu).  With ``treks`` (one trek
+    regulariser or None per problem) the problems run one after the other as ``DagmaLinear(trek_reg=treks[b])``: the
+    lane count is sized for csrc/lin_iter.cu, which a trek regulariser turns off."""
     batch, d, _ = covd.shape
     lam = np.broadcast_to(np.asarray(lambda1.cpu() if isinstance(lambda1, torch.Tensor) else lambda1,
                                      dtype=np.float64), (batch,))
@@ -513,17 +588,21 @@ def _minimize_batch_large(W, covd, lambda1, mu, max_iter, s, lr, *, tol, beta_1,
     stats = np.zeros((batch, 1, 8))
 
     def solve(b):
-        m = DagmaLinear("l2" if Xd is None else "logistic")
+        m = DagmaLinear("l2" if Xd is None else "logistic", trek_reg=treks[b] if treks is not None else None)
         m._fit_from_cov(covd[b], float(lam[b]), T=1, warm_iter=0, max_iter=0, checkpoint=checkpoint,
                         exclude_edges=exclude_edges, include_edges=include_edges,
                         X_dev=Xd[b] if Xd is not None else None)
         _, ok[b] = m.minimize(W_out[b], mu, int(max_iter), s, lr=lr, tol=tol, beta_1=beta_1, beta_2=beta_2)
         stats[b, 0, 0] = m.last_iters
-        stats[b, 0, 1], stats[b, 0, 2] = m._large.last_lr, s
+        stats[b, 0, 1], stats[b, 0, 2] = (m._large.last_lr if m._large is not None else lr), s
         if m.checkpoint_log:
             stats[b, 0, 3:6] = m.checkpoint_log[-1][2:5]
 
-    _run_lanes(batch, d, solve, covd.device, Xd.shape[1] if Xd is not None else None)
+    if treks is not None:
+        for b in range(batch):
+            solve(b)
+    else:
+        _run_lanes(batch, d, solve, covd.device, Xd.shape[1] if Xd is not None else None)
     if isinstance(W, torch.Tensor):
         W.copy_(torch.from_numpy(W_out))
         return W, (torch.from_numpy(ok).to(W.device) if W.is_cuda else ok), (torch.from_numpy(stats).to(W.device) if W.is_cuda else stats)
@@ -531,11 +610,12 @@ def _minimize_batch_large(W, covd, lambda1, mu, max_iter, s, lr, *, tol, beta_1,
     return W, ok, stats
 
 
-def _fit_batch_large(covd, lambda1, *, w_threshold, return_info, Xd=None, **fit_kw):
+def _fit_batch_large(covd, lambda1, *, w_threshold, return_info, Xd=None, treks=None, **fit_kw):
     """``fit_batch`` beyond the on-chip size (d > 64): every problem runs on the multi-CTA engine -- the same code path
     as ``DagmaLinear.fit`` at that size, fed with the covariance instead of the data -- and ``_batch_lanes`` problems
     run concurrently, each on its own stream (for d <= 128 the inner iterations of a problem are one persistent kernel
-    on a handful of SMs)."""
+    on a handful of SMs).  With ``treks`` the problems run one after the other as ``DagmaLinear(trek_reg=treks[b])``
+    (see ``_minimize_batch_large``)."""
     batch, d, _ = covd.shape
     lam = np.broadcast_to(np.asarray(lambda1.cpu() if isinstance(lambda1, torch.Tensor) else lambda1,
                                      dtype=np.float64), (batch,))
@@ -543,14 +623,18 @@ def _fit_batch_large(covd, lambda1, *, w_threshold, return_info, Xd=None, **fit_
     stage_iters, h_fin, sc_fin = [None] * batch, [None] * batch, [None] * batch
 
     def solve(b):
-        m = DagmaLinear("l2" if Xd is None else "logistic")
+        m = DagmaLinear("l2" if Xd is None else "logistic", trek_reg=treks[b] if treks is not None else None)
         kw = dict(fit_kw)
         kw["s"] = list(kw["s"]) if isinstance(kw["s"], (list, tuple)) else kw["s"]
         m._fit_from_cov(covd[b], float(lam[b]), X_dev=Xd[b] if Xd is not None else None, **kw)
         W_raw[b] = m.W_raw
         stage_iters[b], h_fin[b], sc_fin[b] = m.stage_iters, m.h_final, m.score_final
 
-    _run_lanes(batch, d, solve, covd.device, Xd.shape[1] if Xd is not None else None)
+    if treks is not None:
+        for b in range(batch):
+            solve(b)
+    else:
+        _run_lanes(batch, d, solve, covd.device, Xd.shape[1] if Xd is not None else None)
     W_est = W_raw.copy()
     W_est[np.abs(W_est) < w_threshold] = 0
     if not return_info:

@@ -73,6 +73,11 @@ def fit_batch_sharded(X=None, lambda1=0.03, *, cov=None, group=None, solver=None
     if solver is None:
         from .linear import fit_batch as solver          # the B200 path
     kw = dict(fit_kw)
+    if isinstance(kw.get("trek_reg"), (list, tuple)):     # one regulariser per problem: it travels with its problem
+        treks = kw["trek_reg"]
+        if len(treks) != n_problems:
+            raise ValueError(f"fit_batch_sharded: trek_reg has {len(treks)} entries for {n_problems} problems")
+        kw["trek_reg"] = [treks[i] for i in idx]
     if device is not None:
         kw["device"] = device
     local_in = np.asarray(src)[idx] if not isinstance(src, torch.Tensor) else src[torch.as_tensor(idx)]
