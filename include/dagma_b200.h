@@ -123,6 +123,16 @@ int dagma_linear_fit_small_logistic_f64(dagma_stream_t stream, const dagma_small
 int dagma_linear_fit_small_pst_f64(dagma_stream_t stream, const dagma_small_fit_args* args,
                                    const int32_t* pair_off_dev, const int32_t* pairs_dev,
                                    const double* trek_weight_dev, int agg, double eps_inv);
+/* The same for PST(seq="exp", mode="opt") (src/notreks/notreks.py:496-498): F = expm(W o W) by the degree-
+ * DAGMA_PST_EXP_DEGREE Taylor polynomial (Horner) of W o W / 2^DAGMA_PST_EXP_SQUARINGS followed by that many squarings,
+ * H = F^T F, and GT = the top-right block of expm([[W o W, Gt], [0, W o W]]) with Gt = (F (G_H + G_H^T))^T, by the same
+ * algorithm on the two blocks of the block upper-triangular iterates.  Same contract and checks as above; the series
+ * has no eps_inv.  One CTA per problem (one per SM).                                                              */
+#define DAGMA_PST_EXP_DEGREE 18
+#define DAGMA_PST_EXP_SQUARINGS 12
+int dagma_linear_fit_small_pst_exp_f64(dagma_stream_t stream, const dagma_small_fit_args* args,
+                                       const int32_t* pair_off_dev, const int32_t* pairs_dev,
+                                       const double* trek_weight_dev, int agg);
 /* launch geometry chosen for (d): CTAs, threads, dynamic shared memory bytes */
 int dagma_linear_fit_small_geometry(int d, int batch, int* ctas, int* threads, size_t* smem_bytes);
 

@@ -47,6 +47,8 @@ EXPORTS = {
     "dagma_linear_fit_small_logistic_f64": (C.c_int, [C.c_void_p, C.POINTER(SmallFitArgs), C.c_int, C.c_void_p]),
     "dagma_linear_fit_small_pst_f64": (C.c_int, [C.c_void_p, C.POINTER(SmallFitArgs), C.c_void_p, C.c_void_p,
                                                  C.c_void_p, C.c_int, C.c_double]),
+    "dagma_linear_fit_small_pst_exp_f64": (C.c_int, [C.c_void_p, C.POINTER(SmallFitArgs), C.c_void_p, C.c_void_p,
+                                                     C.c_void_p, C.c_int]),
     "dagma_linear_fit_small_geometry": (C.c_int, [C.c_int, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int),
                                                   C.POINTER(C.c_size_t)]),
     "dagma_fit_dmma_residency": (C.c_int, [C.POINTER(C.c_int)]),

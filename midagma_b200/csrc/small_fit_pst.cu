@@ -1,26 +1,42 @@
-// Batched DagmaLinear('l2', trek_reg=PST(seq="inv", mode="opt")).minimize / fit for 1 <= d <= 64: one CTA per
+// Batched DagmaLinear('l2', trek_reg=PST(seq="inv" | "exp", mode="opt")).minimize / fit for 1 <= d <= 64: one CTA per
 // problem runs the whole schedule (stages, retries, back-tracking, checkpoints) -- the trek-regularised sibling of
 // fit_small_dmma_kernel (small_fit_dmma.cu) and fit_small_logistic_kernel (small_fit_logistic.cu), with the same
 // contract (dagma_small_fit_args) and the same reference semantics (src/dagma/linear.py:165-333 inner loop, :441-457
 // stage loop; quirks Q1-Q7 of SURVEY.md 8), plus the PST term of src/dagma/linear.py:224-276 and
-// src/notreks/notreks.py:500-507, 599-619 with the closed-form adjoint of _pst.py:
+// src/notreks/notreks.py:496-507, 599-619 with the closed-form adjoints of _pst.py.  The kernel is a template on the
+// series; everything but the trek block is shared.
 //
+// seq = "inv":
 //   X   = ((1 + eps) I - W o W)^{-1}                (a second block Gauss-Jordan sweep, no domain check)
 //   v_p = H[i_p, j_p],  H = X^T X                   (only the m pair values, each a dot product of two columns of X)
 //   G_S = G_H + G_H^T                               (pair weights: mean 1/m, sum 1, max ties share, lse softmax(v))
 //   GT^T = X^T (X G_S) X^T                          (= (X Gt X)^T with Gt = G_F^T, G_F = X G_S: three DMMA products)
 //   Gobj += weight * 2 W o GT^T;  obj += weight * pst(W) at the checkpoints
 //
-// Mapping (256 threads, ONE CTA per SM -- X, G_S and the product buffer take 102 KB of shared memory next to the 87 KB
-// of the l2 sweep; problems pulled from an atomic work queue, no grid barriers):
+// seq = "exp" (the arithmetic of _pst.PstEngine and oracle/notreks_ref.py, degree-18 Taylor on M = W o W / 2^12 by
+// Horner, then 12 squarings):
+//   F   = expm(W o W):  R1 = I + M / 18;  R1 <- I + (M R1) / j, j = 17..1;  R1 <- R1 R1 (12 times)      (29 products)
+//         (1 / 18 and 1 / j scale as products with the reciprocal, as in _pst.PstEngine)
+//   v_p = H[i_p, j_p],  H = F^T F;  G_S as above;  E = (F G_S)^T / 2^12                                  (1 product)
+//   GT  = top-right block of expm([[W o W, Gt], [0, W o W]]), Gt = (F G_S)^T, without forming the 2d x 2d matrix:
+//         every iterate of the block algorithm is [[R1, R2], [0, R1]], so with R2 = E / 18 at the start
+//         Horner   R1 <- I + (M R1) / j,   R2 <- (M R2 + E R1) / j                                       (51 products)
+//         squaring R1 <- R1 R1,            R2 <- R1 R2 + R2 R1                                           (36 products)
+//         and R2 ends as GT (R1 ends as F again, bit for bit).
+//
+// Mapping (256 threads, ONE CTA per SM -- the trek buffers take 102 KB (inv: X, G_S, a product buffer) or 136 KB (exp:
+// M, R1, G_S / R2, E) of shared memory next to the 87 KB of the l2 sweep; problems pulled from an atomic work queue,
+// no grid barriers):
 //   * sweep 1 inverts M^T = sI - (W o W)^T with the score GEMM cov (I - W) as filler work, as in the l2 kernel; the
 //     gradient without the trek term and the feasibility flag are formed right after it, the former parked in tensor
-//     memory next to the Adam moments, so the registers are free for sweep 2;
+//     memory next to the Adam moments, so the registers are free for the trek block;
+//   * every product accumulates in DMMA registers, then a barrier, then the result is stored in place;
 //   * pair weights are scattered into G_S with shared-memory atomics.  Every contribution to one entry comes from pairs
 //     with the same unordered key {i, j}, whose values are bit-identical (each computed in the order of (min, max)),
 //     so all addends of one entry are equal and their sum does not depend on the order the atomics land in.  The
-//     normalisation (1/m, 1/ties, 1/sum exp) is applied to GT^T as one scalar; for mean / sum G_S is built once per
-//     problem and the pair values are only needed at the checkpoints.
+//     normalisation (1/m, 1/ties, 1/sum exp) is applied to GT^T as one scalar.  inv, mean / sum: G_S is built once
+//     per problem and the pair values are only needed at the checkpoints.  exp: G_S shares its buffer with R2, so it
+//     is rebuilt every iteration (O(m) atomics next to 117 products).
 #include "common.cuh"
 #define DAGMA_SWEEP_JIT_ROWS 1        // the score filler's accumulators need the registers of the row fragments
 #include "small_dmma.cuh"
@@ -30,6 +46,7 @@
 namespace dagma {
 
 constexpr int PS_TMEM_COLS = 256;         // per thread: m, v (64 columns) and the gradient without the trek term (32)
+constexpr int PST_INV = 0, PST_EXP = 1;   // the series of a kernel instantiation
 
 struct PstSmem {                          // offsets in doubles; the sweep's buffers keep the offsets of DmmaSmem
     static constexpr int X = DmmaSmem::total;                 // [64][68] X = ((1 + eps) I - W o W)^{-1}
@@ -39,6 +56,17 @@ struct PstSmem {                          // offsets in doubles; the sweep's buf
     static constexpr size_t bytes = (size_t)total * sizeof(double);
 };
 static_assert(PstSmem::X % 2 == 0, "16-byte alignment of vector accesses");
+
+struct PstExpSmem {                       // seq = "exp": offsets in doubles after the sweep's buffers
+    static constexpr int M = DmmaSmem::total;                 // [64][68] W o W / 2^12
+    static constexpr int R1 = M + DM_DP * DM_LD;              // [64][68] Horner / squaring iterate; F after the forward chain
+    static constexpr int GS = R1 + DM_DP * DM_LD;             // [64][68] G_H + G_H^T, un-normalised; then R2 (-> GT)
+    static constexpr int E = GS + DM_DP * DM_LD;              // [64][68] (F G_S)^T / 2^12
+    static constexpr int total = E + DM_DP * DM_LD;
+    static constexpr size_t bytes = (size_t)total * sizeof(double);
+};
+static_assert(PstExpSmem::M % 2 == 0, "16-byte alignment of vector accesses");
+static_assert(PstExpSmem::bytes + 1024 <= 232448, "one CTA per SM must fit the opt-in shared memory of a block");
 
 // acc = A B over k < 4 nk on DMMA.8x8x4, accumulator ownership of DmmaPos; A(r, k) = TA ? A[k][r] : A[r][k] and
 // B(k, c) = TB ? B[c][k] : B[k][c], both [64][DM_LD].  Warps whose tiles lie outside d x d get zeros.
@@ -94,12 +122,85 @@ __device__ __forceinline__ void scatter_pair(double* GS, int i, int j, double g)
     atomicAdd(GS + j * DM_LD + i, g);       // G_H^T
 }
 
+// u = A1 B1 and t = A1 B2 + A2 B1 in one pass over k (operands as pst_product with TA = TB = false): a step of the
+// coupled exp chain -- Horner (A1, A2, B1, B2) = (M, E, R1, R2), squaring (R1, R2, R1, R2)
+__device__ __forceinline__ void pst_coupled_product(double (&u)[2][4][2], double (&t)[2][4][2], const DmmaPos& ps,
+                                                    const double* A1, const double* A2, const double* B1,
+                                                    const double* B2, int d) {
+#pragma unroll
+    for (int ti = 0; ti < 2; ++ti)
+#pragma unroll
+        for (int tj = 0; tj < 4; ++tj) u[ti][tj][0] = u[ti][tj][1] = t[ti][tj][0] = t[ti][tj][1] = 0.0;
+    if (16 * ps.wr >= d || 32 * ps.wc >= d) return;
+    const int nk = (d + 3) >> 2;
+#pragma unroll 1
+    for (int kb = 0; kb < nk; ++kb) {
+        const int k = 4 * kb + ps.qc;
+        double a1[2], a2[2], b1[4], b2[4];
+#pragma unroll
+        for (int ti = 0; ti < 2; ++ti) {
+            a1[ti] = A1[ps.row(ti) * DM_LD + k];
+            a2[ti] = A2[ps.row(ti) * DM_LD + k];
+        }
+#pragma unroll
+        for (int tj = 0; tj < 4; ++tj) {
+            const int c = 32 * ps.wc + 8 * tj + ps.qr;
+            b1[tj] = B1[k * DM_LD + c];
+            b2[tj] = B2[k * DM_LD + c];
+        }
+#pragma unroll
+        for (int ti = 0; ti < 2; ++ti)
+#pragma unroll
+            for (int tj = 0; tj < 4; ++tj) {
+                dmma(u[ti][tj][0], u[ti][tj][1], a1[ti], b1[tj]);
+                dmma(t[ti][tj][0], t[ti][tj][1], a1[ti], b2[tj]);
+                dmma(t[ti][tj][0], t[ti][tj][1], a2[ti], b1[tj]);
+            }
+    }
+}
+
+// dst = I_d + acc * (1 / j)  (a Horner step of the Taylor polynomial, scaled as _pst.PstEngine scales it: by the
+// reciprocal -- a division sends the many exact zeros of the padded tiles down its slow path; the identity only
+// inside d x d, so the padding stays 0)
+__device__ __forceinline__ void store_horner(double* dst, const double (&acc)[2][4][2], const DmmaPos& ps, int d,
+                                             double rj) {
+#pragma unroll
+    for (int ti = 0; ti < 2; ++ti)
+#pragma unroll
+        for (int tj = 0; tj < 4; ++tj) {
+            const int r = ps.row(ti), c = ps.col(tj);
+            const double i0 = (r == c && r < d) ? 1.0 : 0.0, i1 = (r == c + 1 && r < d) ? 1.0 : 0.0;
+            *reinterpret_cast<double2*>(dst + r * DM_LD + c) = make_double2(i0 + acc[ti][tj][0] * rj,
+                                                                              i1 + acc[ti][tj][1] * rj);
+        }
+}
+
+__device__ __forceinline__ void store_scaled(double* dst, const double (&acc)[2][4][2], const DmmaPos& ps, double rj) {
+#pragma unroll
+    for (int ti = 0; ti < 2; ++ti)
+#pragma unroll
+        for (int tj = 0; tj < 4; ++tj)
+            *reinterpret_cast<double2*>(dst + ps.row(ti) * DM_LD + ps.col(tj)) =
+                make_double2(acc[ti][tj][0] * rj, acc[ti][tj][1] * rj);
+}
+
+// R1 = I_d + M * (1 / 18) (both [64][DM_LD], whole padded square); the start of both Horner chains
+__device__ __forceinline__ void exp_horner_start(double* R1, const double* M, int d, int tid) {
+    constexpr double RDEG = 1.0 / (double)DAGMA_PST_EXP_DEGREE;
+    for (int idx = tid; idx < DM_DP * DM_DP; idx += DM_NT) {
+        const int r = idx >> 6, c = idx & 63;
+        R1[r * DM_LD + c] = ((r == c && r < d) ? 1.0 : 0.0) + M[r * DM_LD + c] * RDEG;
+    }
+}
+
+template <int SEQ>
 __global__ void __launch_bounds__(DM_NT, 1) fit_small_pst_kernel(const dagma_small_fit_args P,
                                                                   const int32_t* __restrict__ pair_off,
                                                                   const int32_t* __restrict__ pairs,
                                                                   const double* __restrict__ trek_weight, int agg,
                                                                   double eps_inv) {
     using S = DmmaSmem;
+    constexpr bool EXP = SEQ == PST_EXP;
     constexpr int NT = DM_NT, LD = DM_LD;
     extern __shared__ __align__(16) double smem[];
     double* ncov = smem + S::ncov;
@@ -107,8 +208,12 @@ __global__ void __launch_bounds__(DM_NT, 1) fit_small_pst_kernel(const dagma_sma
     double* pinfo = smem + S::pinfo;
     double* red = smem + S::red;
     double* Xs = smem + PstSmem::X;
-    double* GS = smem + PstSmem::GS;
+    double* GS = smem + (EXP ? PstExpSmem::GS : PstSmem::GS);
     double* Ps = smem + PstSmem::P;
+    double* Ms = smem + PstExpSmem::M;                       // exp only
+    double* R1s = smem + PstExpSmem::R1;
+    double* Es = smem + PstExpSmem::E;
+    const double* Fs = EXP ? R1s : Xs;                       // the columns the pair values are dot products of
     __shared__ unsigned s_prob;
     __shared__ uint32_t s_tmem;
     // Adam bias correction, kept by one lane (see fit_small_dmma_kernel)
@@ -172,7 +277,7 @@ __global__ void __launch_bounds__(DM_NT, 1) fit_small_pst_kernel(const dagma_sma
         }
         for (int e = tid; e < DM_DP * LD; e += NT) GS[e] = 0.0;
         __syncthreads();
-        if (m > 0 && !pair_agg) {                       // mean / sum: G_S counts the pairs, fixed for the problem
+        if (!EXP && m > 0 && !pair_agg) {               // inv, mean / sum: G_S counts the pairs, fixed for the problem
             for (int p = tid; p < m; p += NT) {
                 const int2 ij = pr[p];
                 scatter_pair(GS, ij.x, ij.y, 1.0);
@@ -362,36 +467,71 @@ __global__ void __launch_bounds__(DM_NT, 1) fit_small_pst_kernel(const dagma_sma
                 tmem_wait_st();
             }
 
-            // ================= PST inv at the current W =================
+            // ================= PST (inv / exp) at the current W =================
             double tval = 0.0, tscale = 0.0;
             double t[2][4][2];
             const bool trek = m > 0 && (at_ckpt || !bad);
             if (trek) {
-                const double dgx = 1.0 + eps_inv;
+                if constexpr (!EXP) {
+                    const double dgx = 1.0 + eps_inv;
 #pragma unroll
-                for (int ti = 0; ti < 2; ++ti) {
-                    const int r = ps.row(ti);
+                    for (int ti = 0; ti < 2; ++ti) {
+                        const int r = ps.row(ti);
 #pragma unroll
-                    for (int tj = 0; tj < 4; ++tj) {
-                        const int c = ps.col(tj);
-                        const double2 w = *reinterpret_cast<const double2*>(Ws + r * LD + c);
-                        const double dg = (r < d) ? dgx : 1.0;
-                        a[ti][tj][0] = ((r == c) ? dg : 0.0) - w.x * w.x;
-                        a[ti][tj][1] = ((r == c + 1) ? dg : 0.0) - w.y * w.y;
+                        for (int tj = 0; tj < 4; ++tj) {
+                            const int c = ps.col(tj);
+                            const double2 w = *reinterpret_cast<const double2*>(Ws + r * LD + c);
+                            const double dg = (r < d) ? dgx : 1.0;
+                            a[ti][tj][0] = ((r == c) ? dg : 0.0) - w.x * w.x;
+                            a[ti][tj][1] = ((r == c + 1) ? dg : 0.0) - w.y * w.y;
+                        }
+                    }
+                    dmma_sweep(a, ps, smem, d, sy);
+                    store_tiles(Xs, a, ps);
+                    if (pair_agg)
+                        for (int idx = tid; idx < d * d; idx += NT) GS[(idx / d) * LD + idx % d] = 0.0;
+                    __syncthreads();
+                } else {
+                    // F = expm(W o W): M = W o W / 2^12, R1 = I + M / 18, Horner j = 17..1, 12 squarings.  G_S is
+                    // cleared meanwhile: its buffer held R2 of the previous iteration (the padding stays 0).
+                    constexpr double SC = 1.0 / (double)(1 << DAGMA_PST_EXP_SQUARINGS);
+                    for (int idx = tid; idx < DM_DP * DM_DP; idx += NT) {
+                        const double w = Ws[(idx >> 6) * LD + (idx & 63)];
+                        Ms[(idx >> 6) * LD + (idx & 63)] = (w * w) * SC;
+                    }
+                    for (int idx = tid; idx < d * d; idx += NT) GS[(idx / d) * LD + idx % d] = 0.0;
+                    __syncthreads();
+                    exp_horner_start(R1s, Ms, d, tid);
+                    __syncthreads();
+#pragma unroll 1
+                    for (int j = DAGMA_PST_EXP_DEGREE - 1; j >= 1; --j) {
+                        pst_product<false, false>(t, ps, Ms, R1s, d);
+                        __syncthreads();
+                        store_horner(R1s, t, ps, d, 1.0 / (double)j);
+                        __syncthreads();
+                    }
+#pragma unroll 1
+                    for (int q = 0; q < DAGMA_PST_EXP_SQUARINGS; ++q) {
+                        pst_product<false, false>(t, ps, R1s, R1s, d);
+                        __syncthreads();
+                        store_tiles(R1s, t, ps);
+                        __syncthreads();
+                    }
+                    if (!pair_agg) {                        // mean / sum: G_S counts the pairs
+                        for (int p = tid; p < m; p += NT) {
+                            const int2 ij = pr[p];
+                            scatter_pair(GS, ij.x, ij.y, 1.0);
+                        }
+                        __syncthreads();
                     }
                 }
-                dmma_sweep(a, ps, smem, d, sy);
-                store_tiles(Xs, a, ps);
-                if (pair_agg)
-                    for (int idx = tid; idx < d * d; idx += NT) GS[(idx / d) * LD + idx % d] = 0.0;
-                __syncthreads();
                 // pair values -> value and the un-normalised pair weights; tscale = weight x normalisation
                 if (!pair_agg) {
                     if (at_ckpt) {
                         double sv = 0.0, z1 = 0.0, z2 = 0.0;
                         for (int p = tid; p < m; p += NT) {
                             const int2 ij = pr[p];
-                            sv += pair_value(Xs, d, ij.x, ij.y);
+                            sv += pair_value(Fs, d, ij.x, ij.y);
                         }
                         block_sum3<NT>(sv, z1, z2, red, tid);
                         tval = (agg == DAGMA_PST_MEAN) ? sv / (double)m : sv;
@@ -401,13 +541,13 @@ __global__ void __launch_bounds__(DM_NT, 1) fit_small_pst_kernel(const dagma_sma
                     double mx = -INFINITY;
                     for (int p = tid; p < m; p += NT) {
                         const int2 ij = pr[p];
-                        mx = fmax(mx, pair_value(Xs, d, ij.x, ij.y));
+                        mx = fmax(mx, pair_value(Fs, d, ij.x, ij.y));
                     }
                     mx = block_max<NT>(mx, red, tid);
                     double se = 0.0, z1 = 0.0, z2 = 0.0;
                     for (int p = tid; p < m; p += NT) {
                         const int2 ij = pr[p];
-                        const double v = pair_value(Xs, d, ij.x, ij.y);
+                        const double v = pair_value(Fs, d, ij.x, ij.y);
                         if (agg == DAGMA_PST_MAX) {
                             if (v == mx) {                  // torch shares the gradient of max() between ties
                                 se += 1.0;
@@ -423,15 +563,61 @@ __global__ void __launch_bounds__(DM_NT, 1) fit_small_pst_kernel(const dagma_sma
                     tval = (agg == DAGMA_PST_MAX) ? mx : mx + log(se);
                     tscale = weight / se;
                 }
-                // GT^T = X^T (X G_S) X^T
-                pst_product<false, false>(t, ps, Xs, GS, d);       // G_F = X G_S
-                store_tiles(Ps, t, ps);
-                __syncthreads();
-                pst_product<false, true>(t, ps, Ps, Xs, d);        // U = G_F X^T
-                __syncthreads();
-                store_tiles(Ps, t, ps);
-                __syncthreads();
-                pst_product<true, false>(t, ps, Xs, Ps, d);        // GT^T = X^T U
+                if constexpr (!EXP) {
+                    // GT^T = X^T (X G_S) X^T
+                    pst_product<false, false>(t, ps, Xs, GS, d);       // G_F = X G_S
+                    store_tiles(Ps, t, ps);
+                    __syncthreads();
+                    pst_product<false, true>(t, ps, Ps, Xs, d);        // U = G_F X^T
+                    __syncthreads();
+                    store_tiles(Ps, t, ps);
+                    __syncthreads();
+                    pst_product<true, false>(t, ps, Xs, Ps, d);        // GT^T = X^T U
+                } else if (!bad) {                          // (an infeasible iterate only needs the value)
+                    constexpr double SC = 1.0 / (double)(1 << DAGMA_PST_EXP_SQUARINGS);
+                    constexpr double RDEG = 1.0 / (double)DAGMA_PST_EXP_DEGREE;
+                    pst_product<false, false>(t, ps, R1s, GS, d);      // G_F = F G_S
+                    __syncthreads();
+                    // E = G_F^T / 2^12 and R2 = E * (1 / 18) (over G_S, dead now); R1 restarts at I + M * (1 / 18)
+#pragma unroll
+                    for (int ti = 0; ti < 2; ++ti)
+#pragma unroll
+                        for (int tj = 0; tj < 4; ++tj)
+#pragma unroll
+                            for (int e = 0; e < 2; ++e) {
+                                const int at = (ps.col(tj) + e) * LD + ps.row(ti);
+                                const double ev = t[ti][tj][e] * SC;
+                                Es[at] = ev;
+                                GS[at] = ev * RDEG;
+                            }
+                    exp_horner_start(R1s, Ms, d, tid);
+                    __syncthreads();
+                    double u[2][4][2];
+#pragma unroll 1
+                    for (int j = DAGMA_PST_EXP_DEGREE - 1; j >= 1; --j) {
+                        pst_coupled_product(u, t, ps, Ms, Es, R1s, GS, d);    // M R1,  M R2 + E R1
+                        __syncthreads();
+                        const double rj = 1.0 / (double)j;
+                        store_horner(R1s, u, ps, d, rj);
+                        store_scaled(GS, t, ps, rj);
+                        __syncthreads();
+                    }
+#pragma unroll 1
+                    for (int q = 0; q < DAGMA_PST_EXP_SQUARINGS; ++q) {
+                        pst_coupled_product(u, t, ps, R1s, GS, R1s, GS, d);   // R1 R1,  R1 R2 + R2 R1
+                        __syncthreads();
+                        store_tiles(R1s, u, ps);
+                        store_tiles(GS, t, ps);
+                        __syncthreads();
+                    }
+                    // GT^T fragments for the Adam epilogue
+#pragma unroll
+                    for (int ti = 0; ti < 2; ++ti)
+#pragma unroll
+                        for (int tj = 0; tj < 4; ++tj)
+#pragma unroll
+                            for (int e = 0; e < 2; ++e) t[ti][tj][e] = GS[(ps.col(tj) + e) * LD + ps.row(ti)];
+                }
             }
 
             if (at_ckpt) {
@@ -570,9 +756,10 @@ __global__ void __launch_bounds__(DM_NT, 1) fit_small_pst_kernel(const dagma_sma
 
 using namespace dagma;
 
-extern "C" int dagma_linear_fit_small_pst_f64(dagma_stream_t stream_, const dagma_small_fit_args* args,
-                                              const int32_t* pair_off_dev, const int32_t* pairs_dev,
-                                              const double* trek_weight_dev, int agg, double eps_inv) {
+namespace {
+
+int check_pst_args(const dagma_small_fit_args* args, const int32_t* pair_off_dev, const int32_t* pairs_dev,
+                   const double* trek_weight_dev, int agg) {
     DAGMA_REQUIRE(args != nullptr, "null args");
     const dagma_small_fit_args& a = *args;
     DAGMA_REQUIRE(a.batch >= 1, "batch must be positive");
@@ -582,23 +769,46 @@ extern "C" int dagma_linear_fit_small_pst_f64(dagma_stream_t stream_, const dagm
     DAGMA_REQUIRE(a.cov_dev && a.w_dev && a.lambda1_dev && a.work_counter_dev, "null device pointer");
     DAGMA_REQUIRE(pair_off_dev && pairs_dev && trek_weight_dev, "null pair / weight pointer");
     DAGMA_REQUIRE(agg >= DAGMA_PST_MEAN && agg <= DAGMA_PST_LSE, "agg must be one of DAGMA_PST_MEAN .. DAGMA_PST_LSE");
-    DAGMA_REQUIRE(eps_inv >= 0.0 && eps_inv < 1e300, "eps_inv must be finite and >= 0");
+    return 0;
+}
+
+// one CTA per SM: 189 KB (inv) or 223 KB (exp) of shared memory; 256 TMEM columns of the 512 of an SM
+template <int SEQ>
+int launch_pst(dagma_stream_t stream_, const dagma_small_fit_args& a, const int32_t* pair_off_dev,
+               const int32_t* pairs_dev, const double* trek_weight_dev, int agg, double eps_inv) {
     DAGMA_REQUIRE(a.ckpt_diag_dev == nullptr, "the PST fit writes no telemetry rows (ckpt_diag_dev must be NULL)");
     DAGMA_REQUIRE(((uintptr_t)pairs_dev & 7u) == 0, "pairs_dev must be 8-byte aligned");
+    const size_t smem = SEQ == PST_EXP ? PstExpSmem::bytes : PstSmem::bytes;
     cudaStream_t stream = (cudaStream_t)stream_;
     int dev = 0, sms = 0;
     DAGMA_CUDA_OK(cudaGetDevice(&dev));
     DAGMA_CUDA_OK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    DAGMA_CUDA_OK(cudaFuncSetAttribute(fit_small_pst_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                       (int)PstSmem::bytes));
-    DAGMA_CUDA_OK(cudaFuncSetAttribute(fit_small_pst_kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
+    DAGMA_CUDA_OK(cudaFuncSetAttribute(fit_small_pst_kernel<SEQ>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                       (int)smem));
+    DAGMA_CUDA_OK(cudaFuncSetAttribute(fit_small_pst_kernel<SEQ>, cudaFuncAttributePreferredSharedMemoryCarveout,
                                        cudaSharedmemCarveoutMaxShared));
-    // one CTA per SM: 189 KB of shared memory; 256 TMEM columns of the 512 of an SM
     long ctas = sms;
     if (ctas > a.batch) ctas = a.batch;
     DAGMA_CUDA_OK(cudaMemsetAsync(a.work_counter_dev, 0, sizeof(uint32_t), stream));
-    fit_small_pst_kernel<<<(int)ctas, DM_NT, PstSmem::bytes, stream>>>(a, pair_off_dev, pairs_dev, trek_weight_dev, agg,
-                                                                        eps_inv);
+    fit_small_pst_kernel<SEQ><<<(int)ctas, DM_NT, smem, stream>>>(a, pair_off_dev, pairs_dev, trek_weight_dev, agg,
+                                                                   eps_inv);
     DAGMA_CUDA_OK(cudaGetLastError());
     return 0;
+}
+
+}  // namespace
+
+extern "C" int dagma_linear_fit_small_pst_f64(dagma_stream_t stream, const dagma_small_fit_args* args,
+                                              const int32_t* pair_off_dev, const int32_t* pairs_dev,
+                                              const double* trek_weight_dev, int agg, double eps_inv) {
+    if (const int rc = check_pst_args(args, pair_off_dev, pairs_dev, trek_weight_dev, agg)) return rc;
+    DAGMA_REQUIRE(eps_inv >= 0.0 && eps_inv < 1e300, "eps_inv must be finite and >= 0");
+    return launch_pst<PST_INV>(stream, *args, pair_off_dev, pairs_dev, trek_weight_dev, agg, eps_inv);
+}
+
+extern "C" int dagma_linear_fit_small_pst_exp_f64(dagma_stream_t stream, const dagma_small_fit_args* args,
+                                                  const int32_t* pair_off_dev, const int32_t* pairs_dev,
+                                                  const double* trek_weight_dev, int agg) {
+    if (const int rc = check_pst_args(args, pair_off_dev, pairs_dev, trek_weight_dev, agg)) return rc;
+    return launch_pst<PST_EXP>(stream, *args, pair_off_dev, pairs_dev, trek_weight_dev, agg, 0.0);
 }

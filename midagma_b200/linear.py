@@ -61,7 +61,8 @@ def _run_small(cov: torch.Tensor, W: torch.Tensor, lambda1: torch.Tensor, mus, s
                want_final=True, want_diag=False, X=None, pst=None) -> SmallFitResult:
     """Launch ``dagma_linear_fit_small_f64`` on device tensors (W is updated in place).  With ``X`` ([batch, n, d]
     device tensor; ``cov`` = its un-centred X^T X / n) the logistic loss: ``dagma_linear_fit_small_logistic_f64``.
-    With ``pst`` (a ``_PstBatch``) the l2 loss plus the PST ``inv`` term: ``dagma_linear_fit_small_pst_f64``."""
+    With ``pst`` (a ``_PstBatch``) the l2 loss plus the PST term: ``dagma_linear_fit_small_pst_f64`` for ``inv``,
+    ``dagma_linear_fit_small_pst_exp_f64`` for ``exp``."""
     _lib.require_device()
     lib = _lib.load()
     batch, d, _ = cov.shape
@@ -98,7 +99,12 @@ def _run_small(cov: torch.Tensor, W: torch.Tensor, lambda1: torch.Tensor, mus, s
     a.ckpt_log = log.data_ptr() if log is not None else None
     a.ckpt_count = cnt.data_ptr() if cnt is not None else None
     a.work_counter = counter.data_ptr()
-    if pst is not None:
+    if pst is not None and pst.eps_inv is None:
+        assert X is None and pst.pair_off.shape[0] == batch + 1
+        _lib.check(lib.dagma_linear_fit_small_pst_exp_f64(_lib.stream_ptr(), C.byref(a), pst.pair_off.data_ptr(),
+                                                          pst.pairs.data_ptr(), pst.weight.data_ptr(), pst.agg),
+                   "dagma_linear_fit_small_pst_exp_f64")
+    elif pst is not None:
         assert X is None and pst.pair_off.shape[0] == batch + 1
         _lib.check(lib.dagma_linear_fit_small_pst_f64(_lib.stream_ptr(), C.byref(a), pst.pair_off.data_ptr(),
                                                       pst.pairs.data_ptr(), pst.weight.data_ptr(), pst.agg,
@@ -242,12 +248,14 @@ _PST_AGGS = {"mean": 0, "sum": 1, "max": 2, "lse": 3}       # DAGMA_PST_* of inc
 
 
 class _PstBatch(typing.NamedTuple):
-    """Pair sets of an on-chip PST ``inv`` batch in the CSR form of ``dagma_linear_fit_small_pst_f64``."""
+    """Pair sets of an on-chip PST batch in the CSR form of ``dagma_linear_fit_small_pst_f64`` (``inv``) /
+    ``dagma_linear_fit_small_pst_exp_f64`` (``exp``).  The series is told by ``eps_inv``: a float for ``inv``, None
+    for ``exp`` (a series without that parameter)."""
     pair_off: torch.Tensor      # [batch + 1] int32
     pairs: torch.Tensor         # [max(total, 1), 2] int32
     weight: torch.Tensor        # [batch] float64
     agg: int
-    eps_inv: float
+    eps_inv: typing.Optional[float]
 
 
 def _trek_batch(trek_reg, batch: int, d: int, loss_type: str, who: str):
@@ -256,8 +264,11 @@ def _trek_batch(trek_reg, batch: int, d: int, loss_type: str, who: str):
 
     Returns None when no problem carries a term that changes W (None, disabled, empty ``I``, mode "log": the reference
     only logs such a value, linear.py:122-133, 251-258).  Otherwise ``(regs, onchip)``: ``regs`` one regulariser per
-    problem; ``onchip`` the host arrays of the PST ``inv`` kernel -- l2, d <= 64, every term PST ``inv`` with one
-    ``agg`` and ``eps_inv`` -- or None when the problems run one after the other as ``DagmaLinear(trek_reg=regs[b])``."""
+    problem; ``onchip`` the host arrays of the on-chip PST kernels -- l2, d <= 64, every term PST ``inv`` with one
+    ``agg`` and ``eps_inv``, or every term PST ``exp`` with one ``agg`` -- or None when the problems run one after the
+    other as ``DagmaLinear(trek_reg=regs[b])``.  ``onchip = (pair_off, pairs, weight, agg, eps_inv)``; ``eps_inv`` is
+    None for ``exp`` (``eps_inv`` and ``K_log`` never reach that series, so problems that differ only in them share a
+    launch)."""
     if trek_reg is None:
         return None
     regs = list(trek_reg) if isinstance(trek_reg, (list, tuple)) else [trek_reg] * batch
@@ -268,8 +279,10 @@ def _trek_batch(trek_reg, batch: int, d: int, loss_type: str, who: str):
     active = [p for p in plans if p is not None]
     if not active:
         return None
-    keys = {(p["kind"], p.get("seq"), p.get("agg"), p.get("eps_inv")) for p in active}
-    if loss_type != "l2" or d > _lib.SMALL_MAX_D or len(keys) != 1 or next(iter(keys))[:2] != ("pst", "inv"):
+    keys = {(p["kind"], p.get("seq"), p.get("agg"), p.get("eps_inv") if p.get("seq") == "inv" else None)
+            for p in active}
+    if (loss_type != "l2" or d > _lib.SMALL_MAX_D or len(keys) != 1
+            or next(iter(keys))[:2] not in (("pst", "inv"), ("pst", "exp"))):
         return regs, None
     _, _, agg, eps_inv = keys.pop()
     off = np.zeros(batch + 1, dtype=np.int64)
@@ -285,7 +298,7 @@ def _trek_batch(trek_reg, batch: int, d: int, loss_type: str, who: str):
     if off[-1] >= 2 ** 31:
         raise ValueError(f"{who}: {off[-1]} trek pairs in one batch (at most 2^31 - 1)")
     pairs = np.concatenate(parts).astype(np.int32) if off[-1] else np.zeros((1, 2), dtype=np.int32)
-    return regs, (off.astype(np.int32), pairs, weight, _PST_AGGS[agg], float(eps_inv))
+    return regs, (off.astype(np.int32), pairs, weight, _PST_AGGS[agg], None if eps_inv is None else float(eps_inv))
 
 
 def _pst_dev(onchip, device) -> _PstBatch:
@@ -303,8 +316,10 @@ def minimize_batch(W, cov, lambda1, mu, max_iter, s, lr, *, tol=1e-6, beta_1=0.9
     (not centred, not modified); ``cov`` is then its X^T X / n and may be None (computed from X).
     ``trek_reg``: one trek regulariser for the batch, or a sequence of one regulariser (or None)
     per problem -- what ``DagmaLinear(loss_type, trek_reg=...)`` would carry.  l2 problems with
-    d <= 64 whose terms are all PST ``seq="inv"`` with one ``agg`` and ``eps_inv`` run in one
-    launch; other regularisers run the problems one after the other through ``DagmaLinear``.
+    d <= 64 whose terms are all PST ``seq="inv"`` with one ``agg`` and ``eps_inv``, or all PST
+    ``seq="exp"`` with one ``agg``, run in one launch; other regularisers (a mix of series,
+    ``log`` / ``binom``, TCC, the logistic loss, d > 64) run the problems one after the other
+    through ``DagmaLinear``.
     Like the reference, ``W`` is updated in place and returned.
     Returns ``(W, success[batch], stage_stats[batch, 1, 8])``."""
     logistic = _logistic_inputs(loss_type, X, "minimize_batch")
@@ -441,7 +456,9 @@ def fit_batch(X=None, lambda1=0.03, *, cov=None, w_threshold=0.3, T=5, mu_init=1
     reference schedule independently (own convergence checks, retries, back-tracking);
     problems are pulled from a device-side work queue by persistent CTAs.
     ``exclude_edges`` / ``include_edges``: tuples of 2-tuples shared by the batch (linear.py:416-426).
-    ``trek_reg``: as in ``minimize_batch`` (one regulariser, or one per problem).
+    ``trek_reg``: as in ``minimize_batch`` (one regulariser, or one per problem); l2 batches at
+    d <= 64 whose terms are all PST ``inv`` (one ``agg`` / ``eps_inv``) or all PST ``exp`` (one
+    ``agg``) run in one launch, other regularisers one problem after the other.
     Returns thresholded ``W_est`` [batch, d, d] as numpy (+ info dict)."""
     logistic = _logistic_inputs(loss_type, X, "fit_batch")
     if logistic and cov is not None:

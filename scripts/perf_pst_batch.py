@@ -1,16 +1,18 @@
-"""Batched PST ``inv`` fits (csrc/small_fit_pst.cu) against the plain l2 batch and the per-problem loop a user has
-without them.
+"""Batched PST ``inv`` or ``exp`` fits (csrc/small_fit_pst.cu) against the plain l2 batch and the per-problem loop a
+user has without them.
 
 Shapes (Gaussian ER2 SEM, seeds from 2000, lambda1 = 0.02): 1024 x (d = 20, n = 500) and 1024 x (d = 64, n = 1000);
-each problem's pair set I is the no-trek pairs of its true graph, PST inv / mean, weight 0.1.  For each shape:
+each problem's pair set I is the no-trek pairs of its true graph, PST ``--seq`` / mean, weight 0.1.  For each shape:
   * minimize_batch(trek_reg=[...]) with tol = 0 (every problem runs every iteration) on device-resident inputs, warmed
     up, timed by CUDA events: problem-iterations/s, achieved FP64 TFLOP/s from the flop model below and its share of the
     FP64 peak measured in the same run (bench.py's yardsticks);
   * the same call without trek_reg (the plain l2 kernel): what the trek term costs;
   * DagmaLinear("l2", trek_reg=...).minimize on 4 of the problems (wall clock ending in a synchronise) and max|dW|.
-Flop model per iteration: 4 d^3 for the l2 iteration (inverse + cov W), 8 d^3 for the trek term (second inverse, three
-products); the pair values (2 d per pair, at checkpoints only for mean) are left out.
-Usage: perf_pst_batch.py --out DIR   (writes DIR/perf_pst_batch.json, nothing else)"""
+Flop model per iteration: 4 d^3 for the l2 iteration (inverse + cov W); for the trek term 8 d^3 with inv (second
+inverse, three products) and 234 d^3 with exp (117 products: 29 for expm, one for F G_S, 87 for the coupled Frechet
+chain); the pair values (2 d per pair, at checkpoints only for inv / mean) are left out.
+Usage: perf_pst_batch.py --out DIR [--seq inv|exp]   (writes DIR/perf_pst_batch.json for inv,
+DIR/perf_pst_exp_batch.json for exp, nothing else)"""
 import argparse
 import json
 import os
@@ -48,8 +50,11 @@ def make_data(batch, d, n):
     return np.stack(Xs), pairs
 
 
-def flop_per_iter(d, trek):
-    return (12.0 if trek else 4.0) * d ** 3
+TREK_FLOP = {"inv": 8.0, "exp": 234.0}       # per d^3 and iteration, see the docstring
+
+
+def flop_per_iter(d, trek, seq="inv"):
+    return (4.0 + (TREK_FLOP[seq] if trek else 0.0)) * d ** 3
 
 
 def device_info():
@@ -95,9 +100,11 @@ def loop(torch, cov, d, regs):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--out", required=True)
+    ap.add_argument("--seq", choices=("inv", "exp"), default="inv")
     args = ap.parse_args()
+    seq = args.seq
     os.makedirs(args.out, exist_ok=True)
-    path = os.path.join(args.out, "perf_pst_batch.json")
+    path = os.path.join(args.out, "perf_pst_batch.json" if seq == "inv" else "perf_pst_exp_batch.json")
     import torch
     from midagma_b200 import _lib
     from midagma_b200.linear import center_cov
@@ -106,8 +113,8 @@ def main():
     _lib.require_device()
     sms = torch.cuda.get_device_properties(0).multi_processor_count
     res = {"device": device_info(), "iterations": ITERS, "tol": 0.0, "mu": MU, "s": S, "lr": LR, "lambda1": LAM,
-           "pst": {"seq": "inv", "agg": "mean", "weight": WEIGHT, "I": "no-trek pairs of the true graph"},
-           "flop_model": "12 d^3 per iteration with the trek term, 4 d^3 without",
+           "pst": {"seq": seq, "agg": "mean", "weight": WEIGHT, "I": "no-trek pairs of the true graph"},
+           "flop_model": f"{TREK_FLOP[seq] + 4:g} d^3 per iteration with the trek term, 4 d^3 without",
            "fp64_peaks_tflops": {k: round(v, 3) for k, v in bench.fp64_peak_tflops(torch, _lib, sms).items()}}
     peak = max(res["fp64_peaks_tflops"].values())
     res["fp64_peak_tflops"] = peak
@@ -119,13 +126,13 @@ def main():
     dump()
     for name, (batch, d, n) in SHAPES.items():
         Xs, pairs = make_data(batch, d, n)
-        regs = [PSTRegularizer(I=p, seq="inv", weight=WEIGHT, mode="opt", kwargs={"agg": "mean"}) for p in pairs]
+        regs = [PSTRegularizer(I=p, seq=seq, weight=WEIGHT, mode="opt", kwargs={"agg": "mean"}) for p in pairs]
         cov = center_cov(torch.as_tensor(Xs).cuda(), center=False)
         Wb, okb, t, iters = batched(torch, cov, d, regs)
         _, okp, tp, itp = batched(torch, cov, d, None)
         Wl, tl, itl = loop(torch, cov, d, regs)
         rate, plain, lrate = iters / t, itp / tp, itl / tl
-        tflops = rate * flop_per_iter(d, True) / 1e12
+        tflops = rate * flop_per_iter(d, True, seq) / 1e12
         r = {"batch": batch, "d": d, "n": n, "mean_pairs": float(np.mean([len(p) for p in pairs])),
              "pst_seconds": t, "pst_problem_iters": iters, "pst_problem_iters_per_s": rate,
              "pst_achieved_fp64_tflops": tflops, "pst_share_of_fp64_peak": tflops / peak,
