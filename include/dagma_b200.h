@@ -133,6 +133,32 @@ int dagma_linear_fit_small_pst_f64(dagma_stream_t stream, const dagma_small_fit_
 int dagma_linear_fit_small_pst_exp_f64(dagma_stream_t stream, const dagma_small_fit_args* args,
                                        const int32_t* pair_off_dev, const int32_t* pairs_dev,
                                        const double* trek_weight_dev, int agg);
+/* The same for TCC(cycle_penalty="spectral", mode="opt") (src/notreks/notreks.py:156-239, 340-378), version
+ * approx_trek_graph or DAG_learning: the Perron pair (rho, u, v) of A = [[W o W, w S], [I, (W o W)^T]] (S the 0/1
+ * indicator of the pairs, duplicates set the same entry) by power steps x <- x' / (||x'|| + eps) from the all-ones
+ * vectors at every evaluation, A never formed:
+ *   Gobj += weight_b * 2 W o [(u1 v1^T + v2 u2^T) / (m (u.v + eps)) - (u1 u1^T + u2 u2^T) / (m (u.u + eps))],
+ *   obj  += weight_b * (rho - u.Bu / (u.u + eps)) / m,   B = [[W o W, 0], [I, (W o W)^T]],
+ * the baseline terms for approx_trek_graph only; m = pair_off_dev[b + 1] - pair_off_dev[b] (duplicates counted).
+ * Per problem: w_dev, eps_dev, n_iter_dev, flags_dev (DAGMA_TCC_* bits).  DAGMA_TCC_POWER: n_iter_dev[b] unshifted
+ * steps.  Otherwise (eig_*): DAGMA_TCC_EIG_WARMUP unshifted steps, rho0 = |v.Av / (v.v + eps)|; if rho0 >
+ * DAGMA_TCC_EIG_NILPOTENT, chunks of DAGMA_TCC_EIG_CHUNK steps on A + DAGMA_TCC_EIG_SHIFT rho0 I until
+ * ||v - v_prev||^2 <= DAGMA_TCC_EIG_TOL^2 or DAGMA_TCC_EIG_MAX_CHUNKS chunks (then status gains DAGMA_ST_PERRON_CAP).
+ * perron_steps_dev [batch] (NULL allowed): power steps of all evaluations of the problem.  Pairs, pair_off_dev,
+ * weight_dev and the other arguments as in dagma_linear_fit_small_pst_f64.  One CTA per problem (one per SM).     */
+#define DAGMA_ST_PERRON_CAP 8            /* some Perron solve hit DAGMA_TCC_EIG_MAX_CHUNKS (not converged) */
+#define DAGMA_TCC_POWER 1                /* flags: method "power" (else eig_numpy / eig_torch)              */
+#define DAGMA_TCC_DAG_LEARNING 2         /* flags: version DAG_learning (else approx_trek_graph)            */
+#define DAGMA_TCC_EIG_WARMUP 8
+#define DAGMA_TCC_EIG_CHUNK 64
+#define DAGMA_TCC_EIG_MAX_CHUNKS 600
+#define DAGMA_TCC_EIG_TOL 1e-13
+#define DAGMA_TCC_EIG_SHIFT 0.25
+#define DAGMA_TCC_EIG_NILPOTENT 1e-200
+int dagma_linear_fit_small_tcc_f64(dagma_stream_t stream, const dagma_small_fit_args* args,
+                                   const int32_t* pair_off_dev, const int32_t* pairs_dev, const double* weight_dev,
+                                   const double* w_dev, const double* eps_dev, const int32_t* n_iter_dev,
+                                   const int32_t* flags_dev, int64_t* perron_steps_dev);
 /* launch geometry chosen for (d): CTAs, threads, dynamic shared memory bytes */
 int dagma_linear_fit_small_geometry(int d, int batch, int* ctas, int* threads, size_t* smem_bytes);
 

@@ -18,6 +18,7 @@ ONCHIP_INV_MAX_D = 128
 DIAG_COLS = 11
 
 ST_OK, ST_OUT_OF_DOMAIN, ST_LR_UNDERFLOW, ST_RETRY_LIMIT = 0, 1, 2, 4
+ST_PERRON_CAP = 8                # TCC batches: some Perron solve hit the chunk cap
 
 
 class SmallFitArgs(C.Structure):
@@ -49,6 +50,9 @@ EXPORTS = {
                                                  C.c_void_p, C.c_int, C.c_double]),
     "dagma_linear_fit_small_pst_exp_f64": (C.c_int, [C.c_void_p, C.POINTER(SmallFitArgs), C.c_void_p, C.c_void_p,
                                                      C.c_void_p, C.c_int]),
+    "dagma_linear_fit_small_tcc_f64": (C.c_int, [C.c_void_p, C.POINTER(SmallFitArgs), C.c_void_p, C.c_void_p,
+                                                 C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                 C.c_void_p]),
     "dagma_linear_fit_small_geometry": (C.c_int, [C.c_int, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int),
                                                   C.POINTER(C.c_size_t)]),
     "dagma_fit_dmma_residency": (C.c_int, [C.POINTER(C.c_int)]),

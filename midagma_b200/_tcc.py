@@ -23,6 +23,10 @@ import torch
 
 from . import _lib
 
+# the schedule of ``PerronSolver.converged``; the on-chip TCC fit (DAGMA_TCC_EIG_* of include/dagma_b200.h) runs the same
+EIG_WARMUP = 8           # unshifted steps from the all-ones vectors
+EIG_NILPOTENT = 1e-200   # |rho| of the warm-up vectors at or below which A is taken as nilpotent
+EIG_SHIFT = 0.25         # the chunks iterate on A + EIG_SHIFT * rho0 I
 EIG_TOL = 1e-13          # ||v_k - v_{k-chunk}|| at which the iterated Perron pair is taken as converged
 EIG_CHUNK = 64
 EIG_MAX_CHUNKS = 600
@@ -54,14 +58,14 @@ class PerronSolver:
 
     def converged(self, A: torch.Tensor, eps: float, square: bool = False) -> int:
         """The Perron pair a dense eigensolver returns, by power steps on A + shift I; returns the iterations used."""
-        self._run(A, square, 0.0, 8, eps, 0)
+        self._run(A, square, 0.0, EIG_WARMUP, eps, 0)
         rho0 = abs(float(self.scal[0].item()))
-        if not rho0 > 1e-200:
+        if not rho0 > EIG_NILPOTENT:
             # nilpotent matrix (e.g. the block matrix at W = 0 with an acyclic pair set): rho = 0, the iterates vanish
             # and every eigenvector choice gives the same (zero) fold-back 2 W o (...) -- nothing to converge to
-            return 8
-        shift = 0.25 * rho0                                     # breaks periodicity, keeps most of the spectral gap
-        total = 8
+            return EIG_WARMUP
+        shift = EIG_SHIFT * rho0                                # breaks periodicity, keeps most of the spectral gap
+        total = EIG_WARMUP
         for _ in range(EIG_MAX_CHUNKS):
             self._prev.copy_(self.v)
             self._run(A, square, shift, EIG_CHUNK, eps, 1)

@@ -1,4 +1,5 @@
-// Batched DagmaLinear('l2', trek_reg=PST(seq="inv" | "exp", mode="opt")).minimize / fit for 1 <= d <= 64: one CTA per
+// Batched DagmaLinear('l2', trek_reg=PST(seq="inv" | "exp", mode="opt") or TCC(cycle_penalty="spectral", mode="opt"))
+// .minimize / fit for 1 <= d <= 64: one CTA per
 // problem runs the whole schedule (stages, retries, back-tracking, checkpoints) -- the trek-regularised sibling of
 // fit_small_dmma_kernel (small_fit_dmma.cu) and fit_small_logistic_kernel (small_fit_logistic.cu), with the same
 // contract (dagma_small_fit_args) and the same reference semantics (src/dagma/linear.py:165-333 inner loop, :441-457
@@ -37,6 +38,18 @@
 //     normalisation (1/m, 1/ties, 1/sum exp) is applied to GT^T as one scalar.  inv, mean / sum: G_S is built once
 //     per problem and the pair values are only needed at the checkpoints.  exp: G_S shares its buffer with R2, so it
 //     is rebuilt every iteration (O(m) atomics next to 117 products).
+//
+// TCC (the arithmetic of _tcc.SpectralTcc / PerronSolver, src/notreks/notreks.py:156-239, 340-378): the Perron pair of
+// A = [[W2, w S], [I, W2^T]], W2 = W o W, by power steps that never form A:
+//     v1' = W2 v1 + w S v2,  v2' = v1 + W2^T v2,  u1' = W2^T u1 + u2,  u2' = w S^T u1 + W2 u2,  x <- x' / (||x'|| + eps)
+//   from the all-ones vectors at every evaluation, with the schedule of PerronSolver (power: n_iter steps; eig: 8 steps,
+//   then chunks of 64 steps on A + rho0 / 4 I until v stops moving, unless rho0 = 0).  Thread t < 128 owns row t of the
+//   v chain, thread 128 + t row t of the u chain; each row is a dot product of length d over W2 or W2^T (both kept in
+//   shared memory, column access) plus the S part, a walk over the set bits of a 64-bit row / column word of S held in
+//   a register.  The squared norms are warp partials summed in warp order: one barrier per step, and every sum has a
+//   fixed order and owner, so a problem gives the same bits alone or anywhere in a batch.  The gradient is the rank-2
+//   fold 2 W o (u1 v1^T + v2 u2^T) / (m (u.v + eps)) (minus the approx_trek_graph baseline), formed entry by entry in
+//   the Adam epilogue; no d x d product.  One solve serves the checkpoint value and the step that follows it.
 #include "common.cuh"
 #define DAGMA_SWEEP_JIT_ROWS 1        // the score filler's accumulators need the registers of the row fragments
 #include "small_dmma.cuh"
@@ -46,7 +59,7 @@
 namespace dagma {
 
 constexpr int PS_TMEM_COLS = 256;         // per thread: m, v (64 columns) and the gradient without the trek term (32)
-constexpr int PST_INV = 0, PST_EXP = 1;   // the series of a kernel instantiation
+constexpr int PST_INV = 0, PST_EXP = 1, TREK_TCC = 2;   // the trek term of a kernel instantiation
 
 struct PstSmem {                          // offsets in doubles; the sweep's buffers keep the offsets of DmmaSmem
     static constexpr int X = DmmaSmem::total;                 // [64][68] X = ((1 + eps) I - W o W)^{-1}
@@ -67,6 +80,198 @@ struct PstExpSmem {                       // seq = "exp": offsets in doubles aft
 };
 static_assert(PstExpSmem::M % 2 == 0, "16-byte alignment of vector accesses");
 static_assert(PstExpSmem::bytes + 1024 <= 232448, "one CTA per SM must fit the opt-in shared memory of a block");
+
+struct TccSmem {                          // TCC: offsets in doubles after the sweep's buffers
+    static constexpr int W2 = DmmaSmem::total;                // [64][68] W o W
+    static constexpr int W2T = W2 + DM_DP * DM_LD;            // [64][68] (W o W)^T
+    static constexpr int X = W2T + DM_DP * DM_LD;             // 2 x [256] iterates: v at 0, u at 128 (rows < 2d used)
+    static constexpr int VP = X + 2 * 256;                    // [128] v before a chunk
+    static constexpr int NRED = VP + 128;                     // 2 x [8] warp partials of the squared norms
+    static constexpr int SRED = NRED + 16;                    // [8][3] warp partials of the Perron scalars
+    static constexpr int DRED = SRED + 24;                    // [8] warp partials of ||v - v_prev||^2
+    static constexpr int SBITS = DRED + 8;                    // [2][64] uint64: rows of S, columns of S
+    static constexpr int total = SBITS + 128;
+    static constexpr size_t bytes = (size_t)total * sizeof(double);
+};
+static_assert(TccSmem::W2 % 2 == 0 && TccSmem::bytes + 1024 <= 232448, "TCC shared memory layout");
+
+// per-problem parameters of the TCC instantiation (the PST ones ignore them)
+struct TccArgs {
+    const double* w;                      // [batch] weight of the S block
+    const double* eps;                    // [batch] eps of the normalisation and the denominators
+    const int32_t* n_iter;                // [batch] steps of method "power"
+    const int32_t* flags;                 // [batch] DAGMA_TCC_* bits
+    long long* perron_steps;              // [batch] power steps of all solves (may be NULL)
+};
+
+__device__ __forceinline__ double warp_sum(double x) {
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) x += __shfl_xor_sync(0xffffffffu, x, off);
+    return x;
+}
+
+// Row rr (< 2d) of A x (form 0) or A^T x (form 1) for a 2d-vector x, A = [[W2, w S], [I, W2^T]].  The rows with an S
+// part (form 0 top: S row i, form 1 bottom: S column i) walk the set bits of sb in increasing order.  B x is form 0
+// with sb = 0.
+__device__ __forceinline__ double tcc_row(int form, int rr, int d, const double* W2, const double* W2T,
+                                          const double* x, unsigned long long sb, double w) {
+    const bool top = rr < d;
+    const int i = top ? rr : rr - d;
+    const bool srow = (form == 0) == top;
+    const double* M = srow ? W2T : W2;                       // M[k][i]: (W2)_{ik} for srow, (W2)_{ki} otherwise
+    const double* xh = x + (top ? 0 : d);
+    const double* xo = x + (top ? d : 0);
+    double acc = 0.0;
+#pragma unroll 4
+    for (int k = 0; k < d; ++k) acc = fma(M[k * DM_LD + i], xh[k], acc);
+    if (!srow) return acc + xo[i];
+    double sacc = 0.0;
+    while (sb) {
+        sacc += xo[__ffsll((long long)sb) - 1];
+        sb &= sb - 1;
+    }
+    return fma(w, sacc, acc);
+}
+
+struct TccResult {
+    double tval;                          // penalty / m
+    double g1, g2;                        // 1 / (m (u.v + eps)), 1 / (m (u.u + eps)) (0 for DAG_learning)
+    const double* V;                      // [256] normalised v (0..2d), u (128..128 + 2d)
+    int steps;
+    bool cap;
+};
+
+// The Perron solve of one evaluation at Ws (PerronSolver.power / .converged, then SpectralTcc.compute / .value).
+// Uniform control flow: every decision reads values all threads computed in the same order.
+__device__ TccResult tcc_perron(double* smem, const double* Ws, int d, int m, double w, double eps, int n_iter,
+                                int flags, unsigned long long sb, int tid) {
+    constexpr int LD = DM_LD;
+    double* W2 = smem + TccSmem::W2;
+    double* W2T = smem + TccSmem::W2T;
+    double* X = smem + TccSmem::X;
+    double* VP = smem + TccSmem::VP;
+    double* nred = smem + TccSmem::NRED;
+    double* sred = smem + TccSmem::SRED;
+    double* dred = smem + TccSmem::DRED;
+    const int chain = tid >> 7, rr = tid & 127, warp = tid >> 5, lane = tid & 31;
+    const bool active = rr < 2 * d;
+    for (int idx = tid; idx < d * d; idx += DM_NT) {
+        const int r = idx / d, c = idx - r * d;
+        const double x = Ws[r * LD + c];
+        W2[r * LD + c] = x * x;
+        W2T[c * LD + r] = x * x;
+    }
+    if (active) X[128 * chain + rr] = 1.0;
+    __syncthreads();
+    int cur = 0;
+    bool unit = true;                     // X[cur] is used as it stands (ones, or normalised vectors)
+    auto inv_norm = [&]() -> double {
+        if (unit) return 1.0;
+        const double* q = nred + 8 * cur + 4 * chain;
+        return 1.0 / (sqrt(((q[0] + q[1]) + q[2]) + q[3]) + eps);
+    };
+    // n steps x <- (A x + shift x) / (||.|| + eps) of both chains (the division deferred to the next reader)
+    auto steps = [&](int n, double shift) {
+#pragma unroll 1
+        for (int k = 0; k < n; ++k) {
+            const double sc = inv_norm();
+            const double* x = X + 256 * cur + 128 * chain;
+            double y = 0.0;
+            if (active) {
+                double acc = tcc_row(chain, rr, d, W2, W2T, x, sb, w);
+                if (shift != 0.0) acc = fma(shift, x[rr], acc);
+                y = acc * sc;
+                X[256 * (cur ^ 1) + 128 * chain + rr] = y;
+            }
+            const double q = warp_sum(y * y);
+            if (lane == 0) nred[8 * (cur ^ 1) + warp] = q;
+            __syncthreads();
+            cur ^= 1;
+            unit = false;
+        }
+    };
+    auto finish = [&]() {                 // normalise in place: X[cur] = v, u
+        const double sc = inv_norm();
+        if (active) X[256 * cur + 128 * chain + rr] *= sc;
+        __syncthreads();
+        unit = true;
+    };
+    double vav = 0.0, vv = 0.0, uv = 0.0, ubu = 0.0, uu = 0.0;
+    auto scalars = [&]() {                // v.Av, v.v, u.v (v chain); u.Bu, u.u (u chain)
+        const double* V = X + 256 * cur;
+        double p0 = 0.0, p1 = 0.0, p2 = 0.0;
+        if (active) {
+            if (chain == 0) {
+                const double vr = V[rr];
+                p0 = vr * tcc_row(0, rr, d, W2, W2T, V, sb, w);
+                p1 = vr * vr;
+                p2 = V[128 + rr] * vr;
+            } else {
+                const double ur = V[128 + rr];
+                p0 = ur * tcc_row(0, rr, d, W2, W2T, V + 128, 0ull, w);
+                p1 = ur * ur;
+            }
+        }
+        p0 = warp_sum(p0);
+        p1 = warp_sum(p1);
+        p2 = warp_sum(p2);
+        if (lane == 0) { sred[3 * warp] = p0; sred[3 * warp + 1] = p1; sred[3 * warp + 2] = p2; }
+        __syncthreads();
+        vav = ((sred[0] + sred[3]) + sred[6]) + sred[9];
+        vv = ((sred[1] + sred[4]) + sred[7]) + sred[10];
+        uv = ((sred[2] + sred[5]) + sred[8]) + sred[11];
+        ubu = ((sred[12] + sred[15]) + sred[18]) + sred[21];
+        uu = ((sred[13] + sred[16]) + sred[19]) + sred[22];
+        __syncthreads();                  // sred is free again
+    };
+    TccResult res;
+    res.cap = false;
+    if (flags & DAGMA_TCC_POWER) {
+        const int n = n_iter > 0 ? n_iter : 0;
+        steps(n, 0.0);
+        finish();
+        scalars();
+        res.steps = n;
+    } else {
+        steps(DAGMA_TCC_EIG_WARMUP, 0.0);
+        finish();
+        scalars();
+        res.steps = DAGMA_TCC_EIG_WARMUP;
+        const double rho0 = fabs(vav / (vv + eps));
+        if (rho0 > DAGMA_TCC_EIG_NILPOTENT) {   // else nilpotent: the warm-up vectors stand (PerronSolver.converged)
+            const double shift = DAGMA_TCC_EIG_SHIFT * rho0;
+            bool conv = false;
+#pragma unroll 1
+            for (int c = 0; c < DAGMA_TCC_EIG_MAX_CHUNKS && !conv; ++c) {
+                if (chain == 0 && active) VP[rr] = X[256 * cur + rr];
+                steps(DAGMA_TCC_EIG_CHUNK, shift);   // (its first barrier orders VP before the reads below)
+                finish();
+                res.steps += DAGMA_TCC_EIG_CHUNK;
+                double df = 0.0;
+                if (chain == 0 && active) {
+                    const double e = X[256 * cur + rr] - VP[rr];
+                    df = e * e;
+                }
+                df = warp_sum(df);
+                if (lane == 0) dred[warp] = df;
+                __syncthreads();
+                const double dn = ((dred[0] + dred[1]) + dred[2]) + dred[3];
+                conv = dn <= DAGMA_TCC_EIG_TOL * DAGMA_TCC_EIG_TOL;
+                __syncthreads();              // dred is free again
+            }
+            res.cap = !conv;
+            scalars();
+        }
+    }
+    const double rm = 1.0 / (double)m;
+    const bool approx = !(flags & DAGMA_TCC_DAG_LEARNING);
+    const double rho = vav / (vv + eps);
+    res.tval = (approx ? rho - ubu / (uu + eps) : rho) * rm;
+    res.g1 = rm / (uv + eps);
+    res.g2 = approx ? rm / (uu + eps) : 0.0;
+    res.V = X + 256 * cur;
+    return res;
+}
 
 // acc = A B over k < 4 nk on DMMA.8x8x4, accumulator ownership of DmmaPos; A(r, k) = TA ? A[k][r] : A[r][k] and
 // B(k, c) = TB ? B[c][k] : B[k][c], both [64][DM_LD].  Warps whose tiles lie outside d x d get zeros.
@@ -198,9 +403,10 @@ __global__ void __launch_bounds__(DM_NT, 1) fit_small_pst_kernel(const dagma_sma
                                                                   const int32_t* __restrict__ pair_off,
                                                                   const int32_t* __restrict__ pairs,
                                                                   const double* __restrict__ trek_weight, int agg,
-                                                                  double eps_inv) {
+                                                                  double eps_inv, const TccArgs tcc) {
     using S = DmmaSmem;
     constexpr bool EXP = SEQ == PST_EXP;
+    constexpr bool TCC = SEQ == TREK_TCC;
     constexpr int NT = DM_NT, LD = DM_LD;
     extern __shared__ __align__(16) double smem[];
     double* ncov = smem + S::ncov;
@@ -226,7 +432,8 @@ __global__ void __launch_bounds__(DM_NT, 1) fit_small_pst_kernel(const dagma_sma
     const int d = P.d;
     const int np = 4 * ((d + 3) >> 2);
     const size_t dd = (size_t)d * d;
-    const bool pair_agg = agg == DAGMA_PST_MAX || agg == DAGMA_PST_LSE;   // G_S depends on the pair values
+    const bool pair_agg = !TCC && (agg == DAGMA_PST_MAX || agg == DAGMA_PST_LSE);   // G_S depends on the pair values
+    unsigned long long* sbits = reinterpret_cast<unsigned long long*>(smem + TccSmem::SBITS);   // TCC only
 
     SweepSync sy{smem_u32(smem + S::mbar), 0u};
     if (tid == 0) mbar_init(sy.bar, NT / 32);
@@ -275,9 +482,31 @@ __global__ void __launch_bounds__(DM_NT, 1) fit_small_pst_kernel(const dagma_sma
             ncov[r * LD + c] = in ? -cov_g[r * d + c] : 0.0;
             Ws[r * LD + c] = in ? W_g[r * d + c] : 0.0;
         }
-        for (int e = tid; e < DM_DP * LD; e += NT) GS[e] = 0.0;
+        double tcc_w = 0.0, tcc_eps = 0.0;
+        int tcc_n_iter = 0, tcc_flags = 0;
+        long long perron_steps = 0;
+        unsigned long long sb = 0;
+        if constexpr (TCC) {
+            tcc_w = tcc.w[b];
+            tcc_eps = tcc.eps[b];
+            tcc_n_iter = tcc.n_iter[b];
+            tcc_flags = tcc.flags[b];
+            if (tid < 128) sbits[tid] = 0ull;
+            __syncthreads();
+            for (int p = tid; p < m; p += NT) {      // S[i][j] = 1 (duplicates set the same bit)
+                const int2 ij = pr[p];
+                atomicOr(sbits + ij.x, 1ull << ij.y);          // row i of S
+                atomicOr(sbits + 64 + ij.y, 1ull << ij.x);     // column j of S
+            }
+            __syncthreads();
+            const int rr = tid & 127;
+            if (tid < 128 && rr < d) sb = sbits[rr];                         // v chain, top rows: S rows
+            if (tid >= 128 && rr >= d && rr < 2 * d) sb = sbits[64 + rr - d];   // u chain, bottom rows: S columns
+        } else {
+            for (int e = tid; e < DM_DP * LD; e += NT) GS[e] = 0.0;
+        }
         __syncthreads();
-        if (!EXP && m > 0 && !pair_agg) {               // inv, mean / sum: G_S counts the pairs, fixed for the problem
+        if (!EXP && !TCC && m > 0 && !pair_agg) {               // inv, mean / sum: G_S counts the pairs, fixed for the problem
             for (int p = tid; p < m; p += NT) {
                 const int2 ij = pr[p];
                 scatter_pair(GS, ij.x, ij.y, 1.0);
@@ -467,11 +696,17 @@ __global__ void __launch_bounds__(DM_NT, 1) fit_small_pst_kernel(const dagma_sma
                 tmem_wait_st();
             }
 
-            // ================= PST (inv / exp) at the current W =================
+            // ================= PST (inv / exp) or TCC at the current W =================
             double tval = 0.0, tscale = 0.0;
             double t[2][4][2];
+            TccResult tr;
             const bool trek = m > 0 && (at_ckpt || !bad);
-            if (trek) {
+            if (TCC && trek) {
+                tr = tcc_perron(smem, Ws, d, m, tcc_w, tcc_eps, tcc_n_iter, tcc_flags, sb, tid);
+                perron_steps += tr.steps;
+                if (tr.cap) status |= DAGMA_ST_PERRON_CAP;
+                tval = tr.tval;
+            } else if (trek) {
                 if constexpr (!EXP) {
                     const double dgx = 1.0 + eps_inv;
 #pragma unroll
@@ -697,7 +932,20 @@ __global__ void __launch_bounds__(DM_NT, 1) fit_small_pst_kernel(const dagma_sma
                     lg.finish();
 #pragma unroll
                     for (int q = 0; q < 8; ++q) go[q] = lg.get(q);
-                    if (trek) {                            // + weight * 2 W o GT^T   (linear.py:251-258)
+                    if (TCC && trek) {                     // + weight * 2 W o (rank-2 fold)   (_tcc.SpectralTcc.compute)
+                        const double* v = tr.V;
+                        const double* u = tr.V + 128;
+                        const int r = ps.row(ti);
+#pragma unroll
+                        for (int q = 0; q < 8; ++q) {
+                            const int c = ps.col(q >> 1) + (q & 1);
+                            if (r < d && c < d) {
+                                const double g = tr.g1 * fma(u[r], v[c], v[d + r] * u[d + c]) -
+                                                 tr.g2 * fma(u[r], u[c], u[d + r] * u[d + c]);
+                                go[q] = fma(twice(w[q]), weight * g, go[q]);
+                            }
+                        }
+                    } else if (trek) {                     // + weight * 2 W o GT^T   (linear.py:251-258)
 #pragma unroll
                         for (int q = 0; q < 8; ++q) go[q] = fma(twice(w[q]), tscale * t[ti][q >> 1][q & 1], go[q]);
                     }
@@ -743,6 +991,7 @@ __global__ void __launch_bounds__(DM_NT, 1) fit_small_pst_kernel(const dagma_sma
         if (tid == 0) {
             if (P.status_dev) P.status_dev[b] = status;
             if (P.ckpt_count_dev) P.ckpt_count_dev[b] = n_ckpt < P.ckpt_log_cap ? n_ckpt : P.ckpt_log_cap;
+            if (TCC && tcc.perron_steps) tcc.perron_steps[b] = perron_steps;
         }
         __syncthreads();
     }
@@ -772,13 +1021,14 @@ int check_pst_args(const dagma_small_fit_args* args, const int32_t* pair_off_dev
     return 0;
 }
 
-// one CTA per SM: 189 KB (inv) or 223 KB (exp) of shared memory; 256 TMEM columns of the 512 of an SM
+// one CTA per SM: 189 KB (inv), 223 KB (exp) or 157 KB (tcc) of shared memory; 256 TMEM columns of the 512 of an SM
 template <int SEQ>
 int launch_pst(dagma_stream_t stream_, const dagma_small_fit_args& a, const int32_t* pair_off_dev,
-               const int32_t* pairs_dev, const double* trek_weight_dev, int agg, double eps_inv) {
+               const int32_t* pairs_dev, const double* trek_weight_dev, int agg, double eps_inv,
+               const TccArgs& tcc = TccArgs{}) {
     DAGMA_REQUIRE(a.ckpt_diag_dev == nullptr, "the PST fit writes no telemetry rows (ckpt_diag_dev must be NULL)");
     DAGMA_REQUIRE(((uintptr_t)pairs_dev & 7u) == 0, "pairs_dev must be 8-byte aligned");
-    const size_t smem = SEQ == PST_EXP ? PstExpSmem::bytes : PstSmem::bytes;
+    const size_t smem = SEQ == PST_EXP ? PstExpSmem::bytes : SEQ == TREK_TCC ? TccSmem::bytes : PstSmem::bytes;
     cudaStream_t stream = (cudaStream_t)stream_;
     int dev = 0, sms = 0;
     DAGMA_CUDA_OK(cudaGetDevice(&dev));
@@ -791,7 +1041,7 @@ int launch_pst(dagma_stream_t stream_, const dagma_small_fit_args& a, const int3
     if (ctas > a.batch) ctas = a.batch;
     DAGMA_CUDA_OK(cudaMemsetAsync(a.work_counter_dev, 0, sizeof(uint32_t), stream));
     fit_small_pst_kernel<SEQ><<<(int)ctas, DM_NT, smem, stream>>>(a, pair_off_dev, pairs_dev, trek_weight_dev, agg,
-                                                                   eps_inv);
+                                                                   eps_inv, tcc);
     DAGMA_CUDA_OK(cudaGetLastError());
     return 0;
 }
@@ -811,4 +1061,15 @@ extern "C" int dagma_linear_fit_small_pst_exp_f64(dagma_stream_t stream, const d
                                                   const double* trek_weight_dev, int agg) {
     if (const int rc = check_pst_args(args, pair_off_dev, pairs_dev, trek_weight_dev, agg)) return rc;
     return launch_pst<PST_EXP>(stream, *args, pair_off_dev, pairs_dev, trek_weight_dev, agg, 0.0);
+}
+
+extern "C" int dagma_linear_fit_small_tcc_f64(dagma_stream_t stream, const dagma_small_fit_args* args,
+                                              const int32_t* pair_off_dev, const int32_t* pairs_dev,
+                                              const double* weight_dev, const double* w_dev, const double* eps_dev,
+                                              const int32_t* n_iter_dev, const int32_t* flags_dev,
+                                              int64_t* perron_steps_dev) {
+    if (const int rc = check_pst_args(args, pair_off_dev, pairs_dev, weight_dev, DAGMA_PST_MEAN)) return rc;
+    DAGMA_REQUIRE(w_dev && eps_dev && n_iter_dev && flags_dev, "null TCC parameter pointer");
+    const TccArgs tcc{w_dev, eps_dev, n_iter_dev, flags_dev, reinterpret_cast<long long*>(perron_steps_dev)};
+    return launch_pst<TREK_TCC>(stream, *args, pair_off_dev, pairs_dev, weight_dev, DAGMA_PST_MEAN, 0.0, tcc);
 }

@@ -58,11 +58,13 @@ class SmallFitResult(typing.NamedTuple):
 
 def _run_small(cov: torch.Tensor, W: torch.Tensor, lambda1: torch.Tensor, mus, ss, iters, *, lr, tol,
                beta1, beta2, checkpoint, retry, mask_exc=None, mask_inc=None, ckpt_log_cap=0,
-               want_final=True, want_diag=False, X=None, pst=None) -> SmallFitResult:
+               want_final=True, want_diag=False, X=None, pst=None, tcc=None) -> SmallFitResult:
     """Launch ``dagma_linear_fit_small_f64`` on device tensors (W is updated in place).  With ``X`` ([batch, n, d]
     device tensor; ``cov`` = its un-centred X^T X / n) the logistic loss: ``dagma_linear_fit_small_logistic_f64``.
     With ``pst`` (a ``_PstBatch``) the l2 loss plus the PST term: ``dagma_linear_fit_small_pst_f64`` for ``inv``,
-    ``dagma_linear_fit_small_pst_exp_f64`` for ``exp``."""
+    ``dagma_linear_fit_small_pst_exp_f64`` for ``exp``.  With ``tcc`` (a ``_TccBatch`` of device tensors) the l2 loss
+    plus the spectral TCC term: ``dagma_linear_fit_small_tcc_f64``; the power steps of each problem are added to
+    ``tcc.perron_steps``."""
     _lib.require_device()
     lib = _lib.load()
     batch, d, _ = cov.shape
@@ -70,7 +72,8 @@ def _run_small(cov: torch.Tensor, W: torch.Tensor, lambda1: torch.Tensor, mus, s
     if T > _lib.MAX_STAGES:
         return _run_small_chunked(cov, W, lambda1, mus, ss, iters, lr=lr, tol=tol, beta1=beta1, beta2=beta2,
                                   checkpoint=checkpoint, retry=retry, mask_exc=mask_exc, mask_inc=mask_inc,
-                                  ckpt_log_cap=ckpt_log_cap, want_final=want_final, want_diag=want_diag, X=X, pst=pst)
+                                  ckpt_log_cap=ckpt_log_cap, want_final=want_final, want_diag=want_diag, X=X, pst=pst,
+                                  tcc=tcc)
     assert cov.is_cuda and W.is_cuda and cov.dtype == torch.float64 and W.dtype == torch.float64
     assert cov.is_contiguous() and W.is_contiguous() and lambda1.is_contiguous()
     dev = cov.device
@@ -99,7 +102,15 @@ def _run_small(cov: torch.Tensor, W: torch.Tensor, lambda1: torch.Tensor, mus, s
     a.ckpt_log = log.data_ptr() if log is not None else None
     a.ckpt_count = cnt.data_ptr() if cnt is not None else None
     a.work_counter = counter.data_ptr()
-    if pst is not None and pst.eps_inv is None:
+    if tcc is not None:
+        assert X is None and pst is None and tcc.pair_off.shape[0] == batch + 1
+        steps = torch.zeros(batch, dtype=torch.int64, device=dev)
+        _lib.check(lib.dagma_linear_fit_small_tcc_f64(_lib.stream_ptr(), C.byref(a), tcc.pair_off.data_ptr(),
+                                                      tcc.pairs.data_ptr(), tcc.weight.data_ptr(), tcc.w.data_ptr(),
+                                                      tcc.eps.data_ptr(), tcc.n_iter.data_ptr(), tcc.flags.data_ptr(),
+                                                      steps.data_ptr()), "dagma_linear_fit_small_tcc_f64")
+        tcc.perron_steps.add_(steps)
+    elif pst is not None and pst.eps_inv is None:
         assert X is None and pst.pair_off.shape[0] == batch + 1
         _lib.check(lib.dagma_linear_fit_small_pst_exp_f64(_lib.stream_ptr(), C.byref(a), pst.pair_off.data_ptr(),
                                                           pst.pairs.data_ptr(), pst.weight.data_ptr(), pst.agg),
@@ -199,6 +210,17 @@ def _warn_retry_limit(status: torch.Tensor) -> None:
                       "restart point, not a converged solution", RuntimeWarning, stacklevel=3)
 
 
+def _warn_perron_cap(status: torch.Tensor) -> None:
+    """One warning per call when a TCC problem's Perron iteration hit the chunk cap, as ``_tcc.PerronSolver.converged``
+    warns for one solve."""
+    n = int(((status & _lib.ST_PERRON_CAP) != 0).sum().item())
+    if n:
+        import warnings
+        warnings.warn(f"{n} problem(s): the Perron iteration of the TCC penalty did not converge in some evaluation "
+                      "(Perron root not simple / tiny spectral gap): the vectors are the last iterate", RuntimeWarning,
+                      stacklevel=3)
+
+
 
 def _as_dev(x, device, dtype=torch.float64) -> torch.Tensor:
     if isinstance(x, torch.Tensor):
@@ -258,33 +280,25 @@ class _PstBatch(typing.NamedTuple):
     eps_inv: typing.Optional[float]
 
 
-def _trek_batch(trek_reg, batch: int, d: int, loss_type: str, who: str):
-    """``trek_reg`` of a batched call, checked without a device: one regulariser for the whole batch or a sequence with
-    one regulariser (or None) per problem, each validated as ``DagmaLinear(trek_reg=...)`` validates it.
+class _TccBatch(typing.NamedTuple):
+    """Pair sets and per-problem parameters of an on-chip TCC batch (``dagma_linear_fit_small_tcc_f64``): numpy arrays
+    from ``_trek_batch``, device tensors after ``_tcc_dev``.  m of problem b = pair_off[b + 1] - pair_off[b]
+    (duplicates counted, as ``SpectralTcc.n_vals``)."""
+    pair_off: typing.Any        # [batch + 1] int32
+    pairs: typing.Any           # [max(total, 1), 2] int32
+    weight: typing.Any          # [batch] float64
+    w: typing.Any               # [batch] float64, weight of the S block
+    eps: typing.Any             # [batch] float64
+    n_iter: typing.Any          # [batch] int32, steps of method "power"
+    flags: typing.Any           # [batch] int32, _TCC_POWER | _TCC_DAG_LEARNING
+    perron_steps: typing.Any = None   # [batch] int64 device tensor: power steps of all solves, summed over launches
 
-    Returns None when no problem carries a term that changes W (None, disabled, empty ``I``, mode "log": the reference
-    only logs such a value, linear.py:122-133, 251-258).  Otherwise ``(regs, onchip)``: ``regs`` one regulariser per
-    problem; ``onchip`` the host arrays of the on-chip PST kernels -- l2, d <= 64, every term PST ``inv`` with one
-    ``agg`` and ``eps_inv``, or every term PST ``exp`` with one ``agg`` -- or None when the problems run one after the
-    other as ``DagmaLinear(trek_reg=regs[b])``.  ``onchip = (pair_off, pairs, weight, agg, eps_inv)``; ``eps_inv`` is
-    None for ``exp`` (``eps_inv`` and ``K_log`` never reach that series, so problems that differ only in them share a
-    launch)."""
-    if trek_reg is None:
-        return None
-    regs = list(trek_reg) if isinstance(trek_reg, (list, tuple)) else [trek_reg] * batch
-    if len(regs) != batch:
-        raise ValueError(f"{who}: trek_reg has {len(regs)} entries for a batch of {batch} problems")
-    plans = [_trek_plan(r) for r in regs]
-    plans = [p if p is not None and p["mode"] == "opt" else None for p in plans]
-    active = [p for p in plans if p is not None]
-    if not active:
-        return None
-    keys = {(p["kind"], p.get("seq"), p.get("agg"), p.get("eps_inv") if p.get("seq") == "inv" else None)
-            for p in active}
-    if (loss_type != "l2" or d > _lib.SMALL_MAX_D or len(keys) != 1
-            or next(iter(keys))[:2] not in (("pst", "inv"), ("pst", "exp"))):
-        return regs, None
-    _, _, agg, eps_inv = keys.pop()
+
+_TCC_POWER, _TCC_DAG_LEARNING = 1, 2           # DAGMA_TCC_* of include/dagma_b200.h
+
+
+def _pair_csr(plans, batch: int, d: int, who: str):
+    """CSR form of the problems' pair sets (None: no pairs) and their weights; negative indices wrapped."""
     off = np.zeros(batch + 1, dtype=np.int64)
     weight = np.zeros(batch)
     parts = []
@@ -298,13 +312,81 @@ def _trek_batch(trek_reg, batch: int, d: int, loss_type: str, who: str):
     if off[-1] >= 2 ** 31:
         raise ValueError(f"{who}: {off[-1]} trek pairs in one batch (at most 2^31 - 1)")
     pairs = np.concatenate(parts).astype(np.int32) if off[-1] else np.zeros((1, 2), dtype=np.int32)
-    return regs, (off.astype(np.int32), pairs, weight, _PST_AGGS[agg], None if eps_inv is None else float(eps_inv))
+    return off.astype(np.int32), pairs, weight
+
+
+def _tcc_batch(plans, batch: int, d: int, who: str) -> typing.Optional[_TccBatch]:
+    """The on-chip TCC plan, or None when some problem's term, resolved as ``DagmaLinear`` resolves it
+    (``_large._trek_setup``), is not spectral approx_trek_graph / DAG_learning with a method the kernel runs."""
+    from . import notreks
+    w, eps = np.ones(batch), np.full(batch, 1e-12)
+    n_iter, flags = np.zeros(batch, dtype=np.int32), np.zeros(batch, dtype=np.int32)
+    for b, p in enumerate(plans):
+        if p is None:
+            continue
+        kw = notreks._tcc_call_args(p["reg"], notreks.FORWARD_TCC_CONFIG)
+        version, method = kw.get("version", "approx_trek_graph"), kw.get("method", "eig_numpy")
+        if (kw.get("cycle_penalty", "spectral") != "spectral" or version not in ("approx_trek_graph", "DAG_learning")
+                or (method == "power" and not 0 <= kw["n_iter"] < 2 ** 31)):
+            return None
+        w[b], eps[b], n_iter[b] = kw["w"], kw["eps"], kw["n_iter"]
+        flags[b] = (_TCC_POWER if method == "power" else 0) | (_TCC_DAG_LEARNING if version == "DAG_learning" else 0)
+    off, pairs, weight = _pair_csr(plans, batch, d, who)
+    return _TccBatch(off, pairs, weight, w, eps, n_iter, flags)
+
+
+def _trek_batch(trek_reg, batch: int, d: int, loss_type: str, who: str):
+    """``trek_reg`` of a batched call, checked without a device: one regulariser for the whole batch or a sequence with
+    one regulariser (or None) per problem, each validated as ``DagmaLinear(trek_reg=...)`` validates it.
+
+    Returns None when no problem carries a term that changes W (None, disabled, empty ``I``, mode "log": the reference
+    only logs such a value, linear.py:122-133, 251-258).  Otherwise ``(regs, onchip)``: ``regs`` one regulariser per
+    problem; ``onchip`` the host arrays of the on-chip PST kernels -- l2, d <= 64, every term PST ``inv`` with one
+    ``agg`` and ``eps_inv``, or every term PST ``exp`` with one ``agg`` -- or None when the problems run one after the
+    other as ``DagmaLinear(trek_reg=regs[b])``.  ``onchip = (pair_off, pairs, weight, agg, eps_inv)``; ``eps_inv`` is
+    None for ``exp`` (``eps_inv`` and ``K_log`` never reach that series, so problems that differ only in them share a
+    launch).  When every term is TCC and resolves to spectral approx_trek_graph / DAG_learning, ``onchip`` is a
+    ``_TccBatch`` (problems with different w, eps, n_iter, method and version share the launch)."""
+    if trek_reg is None:
+        return None
+    regs = list(trek_reg) if isinstance(trek_reg, (list, tuple)) else [trek_reg] * batch
+    if len(regs) != batch:
+        raise ValueError(f"{who}: trek_reg has {len(regs)} entries for a batch of {batch} problems")
+    plans = [_trek_plan(r) for r in regs]
+    plans = [p if p is not None and p["mode"] == "opt" else None for p in plans]
+    active = [p for p in plans if p is not None]
+    if not active:
+        return None
+    keys = {(p["kind"], p.get("seq"), p.get("agg"), p.get("eps_inv") if p.get("seq") == "inv" else None)
+            for p in active}
+    if loss_type == "l2" and d <= _lib.SMALL_MAX_D and keys == {("tcc", None, None, None)}:
+        return regs, _tcc_batch(plans, batch, d, who)
+    if (loss_type != "l2" or d > _lib.SMALL_MAX_D or len(keys) != 1
+            or next(iter(keys))[:2] not in (("pst", "inv"), ("pst", "exp"))):
+        return regs, None
+    _, _, agg, eps_inv = keys.pop()
+    off, pairs, weight = _pair_csr(plans, batch, d, who)
+    return regs, (off, pairs, weight, _PST_AGGS[agg], None if eps_inv is None else float(eps_inv))
 
 
 def _pst_dev(onchip, device) -> _PstBatch:
     off, pairs, weight, agg, eps_inv = onchip
     dev = lambda a: torch.as_tensor(np.ascontiguousarray(a)).to(device)  # noqa: E731
     return _PstBatch(dev(off), dev(pairs), dev(weight), agg, eps_inv)
+
+
+def _tcc_dev(plan: _TccBatch, device) -> _TccBatch:
+    dev = lambda a: torch.as_tensor(np.ascontiguousarray(a)).to(device)  # noqa: E731
+    return _TccBatch(*(dev(a) for a in plan[:7]), torch.zeros(len(plan.weight), dtype=torch.int64, device=device))
+
+
+def _onchip_trek(trek, device) -> dict:
+    """The ``pst=`` / ``tcc=`` argument of ``_run_small`` for a batch that ``_trek_batch`` sends on chip."""
+    if trek is None:
+        return {}
+    if isinstance(trek[1], _TccBatch):
+        return {"tcc": _tcc_dev(trek[1], device)}
+    return {"pst": _pst_dev(trek[1], device)}
 
 
 def minimize_batch(W, cov, lambda1, mu, max_iter, s, lr, *, tol=1e-6, beta_1=0.99, beta_2=0.999,
@@ -317,9 +399,11 @@ def minimize_batch(W, cov, lambda1, mu, max_iter, s, lr, *, tol=1e-6, beta_1=0.9
     ``trek_reg``: one trek regulariser for the batch, or a sequence of one regulariser (or None)
     per problem -- what ``DagmaLinear(loss_type, trek_reg=...)`` would carry.  l2 problems with
     d <= 64 whose terms are all PST ``seq="inv"`` with one ``agg`` and ``eps_inv``, or all PST
-    ``seq="exp"`` with one ``agg``, run in one launch; other regularisers (a mix of series,
-    ``log`` / ``binom``, TCC, the logistic loss, d > 64) run the problems one after the other
-    through ``DagmaLinear``.
+    ``seq="exp"`` with one ``agg``, or all spectral TCC (``approx_trek_graph`` / ``DAG_learning``
+    as ``DagmaLinear`` resolves them, any mix of w / eps / n_iter / method), run in one launch;
+    other regularisers (a mix of series or of PST and TCC, ``log`` / ``binom``, the other TCC
+    versions, the logistic loss, d > 64) run the problems one after the other through
+    ``DagmaLinear``.
     Like the reference, ``W`` is updated in place and returned.
     Returns ``(W, success[batch], stage_stats[batch, 1, 8])``."""
     logistic = _logistic_inputs(loss_type, X, "minimize_batch")
@@ -345,7 +429,8 @@ def minimize_batch(W, cov, lambda1, mu, max_iter, s, lr, *, tol=1e-6, beta_1=0.9
     mask_exc, mask_inc = _batch_masks(exclude_edges, include_edges, d, device)
     res = _run_small(covd, Wd, lam, [mu], [s], [int(max_iter)], lr=lr, tol=tol, beta1=beta_1, beta2=beta_2,
                      checkpoint=checkpoint, retry=False, want_final=False, mask_exc=mask_exc, mask_inc=mask_inc, X=Xd,
-                     pst=_pst_dev(trek[1], device) if trek is not None else None)
+                     **_onchip_trek(trek, device))
+    _warn_perron_cap(res.status)
     ok = (res.status & _lib.ST_OUT_OF_DOMAIN) == 0
     if on_device:
         if Wd is not W:
@@ -457,9 +542,11 @@ def fit_batch(X=None, lambda1=0.03, *, cov=None, w_threshold=0.3, T=5, mu_init=1
     problems are pulled from a device-side work queue by persistent CTAs.
     ``exclude_edges`` / ``include_edges``: tuples of 2-tuples shared by the batch (linear.py:416-426).
     ``trek_reg``: as in ``minimize_batch`` (one regulariser, or one per problem); l2 batches at
-    d <= 64 whose terms are all PST ``inv`` (one ``agg`` / ``eps_inv``) or all PST ``exp`` (one
-    ``agg``) run in one launch, other regularisers one problem after the other.
-    Returns thresholded ``W_est`` [batch, d, d] as numpy (+ info dict)."""
+    d <= 64 whose terms are all PST ``inv`` (one ``agg`` / ``eps_inv``), all PST ``exp`` (one
+    ``agg``) or all spectral TCC (``approx_trek_graph`` / ``DAG_learning``) run in one launch,
+    other regularisers one problem after the other.
+    Returns thresholded ``W_est`` [batch, d, d] as numpy (+ info dict; an on-chip TCC batch adds
+    ``perron_steps`` [batch], the power steps of all Perron solves of each problem)."""
     logistic = _logistic_inputs(loss_type, X, "fit_batch")
     if logistic and cov is not None:
         raise ValueError("fit_batch(loss_type='logistic') takes X only: the covariance is computed from it")
@@ -494,10 +581,11 @@ def fit_batch(X=None, lambda1=0.03, *, cov=None, w_threshold=0.3, T=5, mu_init=1
     iters = [int(max_iter) if i == T - 1 else int(warm_iter) for i in range(T)]
     Wd = torch.zeros(batch, d, d, dtype=torch.float64, device=device)
     mask_exc, mask_inc = _batch_masks(exclude_edges, include_edges, d, device)
+    onchip = _onchip_trek(trek, device)
     res = _run_small(covd, Wd, lam, mus, ss[:T], iters, lr=lr, tol=tol, beta1=beta_1, beta2=beta_2,
-                     checkpoint=checkpoint, retry=True, mask_exc=mask_exc, mask_inc=mask_inc, X=Xd,
-                     pst=_pst_dev(trek[1], device) if trek is not None else None)
+                     checkpoint=checkpoint, retry=True, mask_exc=mask_exc, mask_inc=mask_inc, X=Xd, **onchip)
     _warn_retry_limit(res.status)
+    _warn_perron_cap(res.status)
     W_raw = res.W.cpu().numpy()
     W_est = W_raw.copy()
     W_est[np.abs(W_est) < w_threshold] = 0
@@ -508,6 +596,8 @@ def fit_batch(X=None, lambda1=0.03, *, cov=None, w_threshold=0.3, T=5, mu_init=1
     info = {"W_raw": W_raw, "status": res.status.cpu().numpy(), "stage_iters": stats[:, :, 0].astype(np.int64),
             "stage_stats": stats, "h_final": fin[:, 0], "score_final": fin[:, 1],
             "total_iters": int(stats[:, :, 0].sum())}
+    if "tcc" in onchip:
+        info["perron_steps"] = onchip["tcc"].perron_steps.cpu().numpy()
     return W_est, info
 
 

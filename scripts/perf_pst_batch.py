@@ -1,5 +1,5 @@
-"""Batched PST ``inv`` or ``exp`` fits (csrc/small_fit_pst.cu) against the plain l2 batch and the per-problem loop a
-user has without them.
+"""Batched PST ``inv`` / ``exp`` or spectral TCC fits (csrc/small_fit_pst.cu) against the plain l2 batch and the
+per-problem loop a user has without them.
 
 Shapes (Gaussian ER2 SEM, seeds from 2000, lambda1 = 0.02): 1024 x (d = 20, n = 500) and 1024 x (d = 64, n = 1000);
 each problem's pair set I is the no-trek pairs of its true graph, PST ``--seq`` / mean, weight 0.1.  For each shape:
@@ -11,8 +11,13 @@ each problem's pair set I is the no-trek pairs of its true graph, PST ``--seq`` 
 Flop model per iteration: 4 d^3 for the l2 iteration (inverse + cov W); for the trek term 8 d^3 with inv (second
 inverse, three products) and 234 d^3 with exp (117 products: 29 for expm, one for F G_S, 87 for the coupled Frechet
 chain); the pair values (2 d per pair, at checkpoints only for inv / mean) are left out.
-Usage: perf_pst_batch.py --out DIR [--seq inv|exp]   (writes DIR/perf_pst_batch.json for inv,
-DIR/perf_pst_exp_batch.json for exp, nothing else)"""
+--seq tcc: TCCRegularizer(I, weight 0.1) with the reference's dispatch (spectral, approx_trek_graph, eig: the Perron
+pair iterated until it stops moving).  Its cost is the number of power steps, a chain of latency-bound steps, so no flop
+model or FP64 share is reported; instead the mean power steps per Perron solve, from the kernel's perron_steps counter of
+an untimed repeat of the batched call (the kernel is deterministic) over its solves (iterations + the final checkpoint
++ back-tracking steps per problem).
+Usage: perf_pst_batch.py --out DIR [--seq inv|exp|tcc]   (writes DIR/perf_pst_batch.json for inv,
+DIR/perf_pst_exp_batch.json for exp, DIR/perf_tcc_batch.json for tcc, nothing else)"""
 import argparse
 import json
 import os
@@ -79,6 +84,21 @@ def batched(torch, cov, d, regs):
     return W.cpu().numpy(), ok.cpu().numpy(), t, float(st[:, 0, 0].sum().item())
 
 
+def perron_steps(torch, cov, d, regs):
+    """Mean power steps per Perron solve of the batched call (an untimed repeat through its launcher)."""
+    from midagma_b200.linear import _run_small, _tcc_dev, _trek_batch
+    batch = cov.shape[0]
+    W = torch.zeros(batch, d, d, dtype=torch.float64, device="cuda")
+    tcc = _tcc_dev(_trek_batch(regs, batch, d, "l2", "perf")[1], "cuda")
+    lam = torch.full((batch,), LAM, dtype=torch.float64, device="cuda")
+    res = _run_small(cov, W, lam, [MU], [S], [ITERS], lr=LR, tol=0.0, beta1=0.99, beta2=0.999, checkpoint=CKPT,
+                     retry=False, want_final=False, tcc=tcc)
+    st = res.stage_stats.cpu().numpy()
+    steps = tcc.perron_steps.cpu().numpy()
+    solves = st[:, 0, 0] + 1 + st[:, 0, 7]
+    return float(steps.sum() / solves.sum()), int(steps.max()), int(((res.status.cpu().numpy() & 8) != 0).sum())
+
+
 def loop(torch, cov, d, regs):
     from midagma_b200 import DagmaLinear
     Ws, t_total, iters = [], 0.0, 0
@@ -100,24 +120,30 @@ def loop(torch, cov, d, regs):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--out", required=True)
-    ap.add_argument("--seq", choices=("inv", "exp"), default="inv")
+    ap.add_argument("--seq", choices=("inv", "exp", "tcc"), default="inv")
     args = ap.parse_args()
     seq = args.seq
+    tcc = seq == "tcc"
     os.makedirs(args.out, exist_ok=True)
-    path = os.path.join(args.out, "perf_pst_batch.json" if seq == "inv" else "perf_pst_exp_batch.json")
+    path = os.path.join(args.out, {"inv": "perf_pst_batch.json", "exp": "perf_pst_exp_batch.json",
+                                   "tcc": "perf_tcc_batch.json"}[seq])
     import torch
     from midagma_b200 import _lib
     from midagma_b200.linear import center_cov
-    from midagma_b200.notreks import PSTRegularizer
+    from midagma_b200.notreks import PSTRegularizer, TCCRegularizer
     import bench
     _lib.require_device()
     sms = torch.cuda.get_device_properties(0).multi_processor_count
-    res = {"device": device_info(), "iterations": ITERS, "tol": 0.0, "mu": MU, "s": S, "lr": LR, "lambda1": LAM,
-           "pst": {"seq": seq, "agg": "mean", "weight": WEIGHT, "I": "no-trek pairs of the true graph"},
-           "flop_model": f"{TREK_FLOP[seq] + 4:g} d^3 per iteration with the trek term, 4 d^3 without",
-           "fp64_peaks_tflops": {k: round(v, 3) for k, v in bench.fp64_peak_tflops(torch, _lib, sms).items()}}
-    peak = max(res["fp64_peaks_tflops"].values())
-    res["fp64_peak_tflops"] = peak
+    res = {"device": device_info(), "iterations": ITERS, "tol": 0.0, "mu": MU, "s": S, "lr": LR, "lambda1": LAM}
+    if tcc:
+        res["tcc"] = {"weight": WEIGHT, "I": "no-trek pairs of the true graph",
+                      "dispatch": "reference default: spectral, approx_trek_graph, eig (converged Perron pair)"}
+    else:
+        res.update({"pst": {"seq": seq, "agg": "mean", "weight": WEIGHT, "I": "no-trek pairs of the true graph"},
+                    "flop_model": f"{TREK_FLOP[seq] + 4:g} d^3 per iteration with the trek term, 4 d^3 without",
+                    "fp64_peaks_tflops": {k: round(v, 3) for k, v in bench.fp64_peak_tflops(torch, _lib, sms).items()}})
+        peak = max(res["fp64_peaks_tflops"].values())
+        res["fp64_peak_tflops"] = peak
 
     def dump():
         with open(path, "w") as f:
@@ -126,23 +152,32 @@ def main():
     dump()
     for name, (batch, d, n) in SHAPES.items():
         Xs, pairs = make_data(batch, d, n)
-        regs = [PSTRegularizer(I=p, seq=seq, weight=WEIGHT, mode="opt", kwargs={"agg": "mean"}) for p in pairs]
+        if tcc:
+            regs = [TCCRegularizer(I=p, weight=WEIGHT, mode="opt") for p in pairs]
+        else:
+            regs = [PSTRegularizer(I=p, seq=seq, weight=WEIGHT, mode="opt", kwargs={"agg": "mean"}) for p in pairs]
         cov = center_cov(torch.as_tensor(Xs).cuda(), center=False)
         Wb, okb, t, iters = batched(torch, cov, d, regs)
         _, okp, tp, itp = batched(torch, cov, d, None)
         Wl, tl, itl = loop(torch, cov, d, regs)
         rate, plain, lrate = iters / t, itp / tp, itl / tl
-        tflops = rate * flop_per_iter(d, True, seq) / 1e12
+        key = "tcc" if tcc else "pst"
         r = {"batch": batch, "d": d, "n": n, "mean_pairs": float(np.mean([len(p) for p in pairs])),
-             "pst_seconds": t, "pst_problem_iters": iters, "pst_problem_iters_per_s": rate,
-             "pst_achieved_fp64_tflops": tflops, "pst_share_of_fp64_peak": tflops / peak,
-             "pst_failed_problems": int((~okb).sum()),
-             "plain_seconds": tp, "plain_problem_iters_per_s": plain,
-             "plain_achieved_fp64_tflops": plain * flop_per_iter(d, False) / 1e12,
-             "trek_cost_factor": plain / rate,
-             "loop_problems": LOOP_PROBLEMS, "loop_seconds": tl, "loop_problem_iters_per_s": lrate,
-             "speedup_vs_loop": rate / lrate,
-             "parity_max_abs_dW_loop_vs_batched": float(np.abs(Wl - Wb[:LOOP_PROBLEMS]).max())}
+             f"{key}_seconds": t, f"{key}_problem_iters": iters, f"{key}_problem_iters_per_s": rate}
+        if tcc:
+            mean_steps, max_steps, capped = perron_steps(torch, cov, d, regs)
+            r.update({"mean_power_steps_per_solve": mean_steps, "max_power_steps_per_problem": max_steps,
+                      "problems_with_capped_solve": capped})
+        else:
+            tflops = rate * flop_per_iter(d, True, seq) / 1e12
+            r.update({"pst_achieved_fp64_tflops": tflops, "pst_share_of_fp64_peak": tflops / peak})
+        r.update({f"{key}_failed_problems": int((~okb).sum()),
+                  "plain_seconds": tp, "plain_problem_iters_per_s": plain,
+                  "plain_achieved_fp64_tflops": plain * flop_per_iter(d, False) / 1e12,
+                  "trek_cost_factor": plain / rate,
+                  "loop_problems": LOOP_PROBLEMS, "loop_seconds": tl, "loop_problem_iters_per_s": lrate,
+                  "speedup_vs_loop": rate / lrate,
+                  "parity_max_abs_dW_loop_vs_batched": float(np.abs(Wl - Wb[:LOOP_PROBLEMS]).max())})
         res[f"shape_{name}"] = r
         print(name, json.dumps(r), flush=True)
         dump()
